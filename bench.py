@@ -3,6 +3,7 @@
 perturbed transmon plants).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload transmon_h16] [--members-total 65536 | --members M]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the CPU path (oracle port of the reference) on the host cores
 
 One "step" = one pass of the whole closed loop (all MPC steps of mpc.py:128-304) over this rank's shard of the
@@ -30,6 +31,7 @@ if ROOT not in sys.path:
 
 METRIC = 'closed-loop MPC trajectories/s'
 UNIT = 'trajectories/s'
+DUMP_SEED = 20220113        # member sample of --dump-outputs
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -210,7 +212,7 @@ class Runner:
         cfg = self.cfg
         self.n_total, self.world = n_total, world
         lo, hi = shard_bounds(n_total, rank, world)
-        self.n = hi - lo
+        self.lo, self.n = lo, hi - lo
         self.ens, _ = maker(n_total, lo=lo, hi=hi)           # this rank's block of the seeded draw, nothing else
         model = cfg['model']
         if cfg.get('per_member_models'):
@@ -244,6 +246,23 @@ class Runner:
                 allreduce_histogram(self.hist)
         return res
 
+    def outputs(self, res, max_members=4096, budget=60 << 20):
+        """What a resident pass hands its caller, as float64 host arrays: every field of the EnsembleResult (complex
+        arrays with a trailing (real, imag) axis) and the fidelity histogram.  Per-member arrays are taken at a fixed,
+        seeded sample of this rank's members, whose global indices are `members`, so that the whole stays within
+        `budget` bytes at any ensemble size while two builds can be compared member for member."""
+        torch = self.torch
+        fields = {k: getattr(res, k) for k in res.__slots__ if getattr(res, k) is not None}
+        per_member = 8 + sum(8 * (2 if v.is_complex() else 1) * v[0].numel() for v in fields.values())
+        k = min(self.n, max_members, (budget - 8 * self.hist.numel()) // per_member)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(self.n, k, replace=False))
+        sel = torch.from_numpy(idx).to(self.hist.device)
+        out = {'members': (self.lo + idx).astype(np.float64), 'fidelity_histogram': self.hist.double().cpu().numpy()}
+        for name, v in fields.items():
+            v = v.index_select(0, sel)
+            out[name] = (torch.view_as_real(v) if v.is_complex() else v).double().cpu().numpy()
+        return out
+
     def e2e_pass(self):
         """The call a user makes: host buffers in, numpy results (xs, us, fidelity, exit codes, counters) out."""
         cfg = self.cfg
@@ -265,13 +284,13 @@ def timed(fn, steps, flush, world, dist):
         if world > 1:
             dist.barrier()
             torch.cuda.synchronize()
-    total_ms, per = 0.0, []
+    total_ms, per, last = 0.0, [], None
     for _ in range(steps):
         flush.fill_(1)
         sync_all()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        fn()
+        last = fn()
         e1.record()
         sync_all()
         per.append(e0.elapsed_time(e1))
@@ -279,15 +298,17 @@ def timed(fn, steps, flush, world, dist):
     t = torch.tensor([total_ms], dtype=torch.float64, device='cuda')
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    return float(t.item()), per
+    return float(t.item()), per, last
 
 
-def measure(run, steps, warmup, flush, world, dist, fp64_peak=None, e2e=True, kernel_passes=None):
-    """value / kernel time / roofline of one Runner; returns a dict."""
+def measure(run, steps, warmup, flush, world, dist, fp64_peak=None, e2e=True, kernel_passes=None, keep_outputs=False):
+    """value / kernel time / roofline of one Runner; returns a dict (with keep_outputs, 'outputs' holds
+    Runner.outputs() of the last timed pass)."""
     import torch
     for _ in range(warmup):
         run.resident_pass()
-    total_ms, _ = timed(run.resident_pass, steps, flush, world, dist)
+    total_ms, _, last = timed(run.resident_pass, steps, flush, world, dist)
+    outputs = run.outputs(last) if keep_outputs else None      # before the next pass overwrites the plan's buffers
     res = run.resident_pass()
     torch.cuda.synchronize()
     counters = res.counters.cpu().numpy()
@@ -314,13 +335,13 @@ def measure(run, steps, warmup, flush, world, dist, fp64_peak=None, e2e=True, ke
     out = dict(value=run.n_total * steps / (total_ms * 1e-3), ms_per_step=total_ms / steps, kernel_ms=kernel_ms,
                flops=flops, per_unit=per_unit, qp_total=qp_total, qp_all=qp_all, counters=counters, qp_count=qp_count,
                exit_codes=exit_codes, fid=fid, members_not_exit0_all_ranks=int(bad_all),
-               achieved_tflops=flops / (kernel_ms * 1e-3) / 1e12)
+               achieved_tflops=flops / (kernel_ms * 1e-3) / 1e12, outputs=outputs)
     if fp64_peak:
         out['frac'] = out['achieved_tflops'] / fp64_peak
     if e2e:
         r = run.e2e_pass()                                  # untimed: first use of the pinned staging buffers
         e2e_steps = max(2, min(steps, 3))
-        e2e_ms, per = timed(run.e2e_pass, e2e_steps, flush, world, dist)
+        e2e_ms, per, _ = timed(run.e2e_pass, e2e_steps, flush, world, dist)
         h2d, d2h = run.e2e_bytes(r)
         out['e2e'] = {'value': run.n_total * e2e_steps / (e2e_ms * 1e-3), 'unit': UNIT, 'ms_per_pass': per,
                       'h2d_bytes_per_step': h2d, 'd2h_bytes_per_step': d2h,
@@ -377,7 +398,15 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip extra.weak / extra.workloads')
     ap.add_argument('--admm-first', action='store_true',
                     help='always run an ADMM block before the active-set rounds (m4q_qp_settings.admm_first)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed pass computed as DIR/<name>.npy: a seeded sample of the members of '
+                         'rank 0 (with --gpus N > 1 only the first 1/N of the ensemble), their global indices in '
+                         'members.npy, and the fidelity histogram of the whole ensemble')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs is not None and args.impl != 'b200':
+        ap.error('--dump-outputs records the outputs of the b200 path')
     weak = args.members is not None
     if weak:
         args.members_total = args.members * args.gpus
@@ -408,9 +437,14 @@ def main():
         run.resident_pass()
     sampler = ClockSampler(local)
     sampler.start()
-    m = measure(run, args.steps, 0, flush, world, dist, fp64_peak)
+    dump = args.dump_outputs is not None and rank == 0
+    m = measure(run, args.steps, 0, flush, world, dist, fp64_peak, keep_outputs=dump)
     sampler.stop_flag.set()
     sampler.join()
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in m['outputs'].items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), arr)
     counters, qp_count, exit_codes, fid = m['counters'], m['qp_count'], m['exit_codes'], m['fid']
     res_bytes = m['e2e']['h2d_bytes_per_step'] + m['e2e']['d2h_bytes_per_step']
 

@@ -1,12 +1,14 @@
 """CPU tests of the oracle (oracle/restate.py, oracle/admm_model.py) against the fixtures generated from the
 reference's own code (oracle/make_golden.py).  No GPU, no /root/reference needed."""
+import itertools
+import math
 import os
 
 import numpy as np
 import pytest
 
 from oracle import restate as rs, admm_model as am, refshim
-from mpc4quantum_b200 import systems
+from mpc4quantum_b200 import linearize, systems
 from conftest import load_golden
 
 
@@ -128,10 +130,53 @@ def test_loop_quirks_are_exercised_by_fixture():
     assert np.abs(rs.proj_coupled(rs.lift_coupled(x1)) - x1).max() < 1e-12
 
 
-@pytest.mark.skipif(not refshim.available(), reason='reference tree only exists in the build container')
-def test_shim_runs_reference_functions():
-    lin = refshim.module('linearize')
-    assert [list(p) for p in lin.create_power_list(2, 2)] == rs.power_table(2, 2).tolist()
+def _reference_monomial_order(L, dt, order, blocks, rng):
+    """The monomial of each block of the reference's discretize_homogeneous output, read off the blocks themselves: the
+    order-k Taylor polynomial of exp((L0 + sum u_i L_i) dt), formed by matrix powers, is sum_b phi_b(u) blocks[b], so a
+    least-squares fit at random u gives phi_b(u) for every block, and each phi_b is matched to one exponent tuple."""
+    m = len(L) - 1
+    basis = blocks.reshape(len(blocks), -1).T
+    us = rng.uniform(-1, 1, size=(3 * len(blocks), m))
+    phi = []
+    for u in us:
+        G = (L[0] + sum(ui * Li for ui, Li in zip(u, L[1:]))) * dt
+        T = sum(np.linalg.matrix_power(G, j) / math.factorial(j) for j in range(order + 1)).reshape(-1)
+        x, _, rank, _ = np.linalg.lstsq(basis, T, rcond=None)
+        assert rank == len(blocks) and np.abs(basis @ x - T).max() < 1e-12
+        phi.append(x)
+    phi = np.array(phi)
+    candidates = [e for e in itertools.product(range(order + 1), repeat=m) if sum(e) <= order]
+    found = []
+    for b in range(len(blocks)):
+        err = [np.abs(phi[:, b] - np.prod(us ** np.array(e), axis=1)).max() for e in candidates]
+        assert min(err) < 1e-10, (b, min(err))
+        found.append(list(candidates[int(np.argmin(err))]))
+    return found
+
+
+def test_shim_runs_reference_functions(unit_golden):
+    """The control-monomial order of the reference (linearize.py:92-116) against power_table and the package's
+    create_power_list, for dim_u = 1, 2, 3 and orders up to 3.  The order is recovered from the reference's own
+    discretisation blocks (tests/golden/unit.npz); where the reference tree is present, also through the shim."""
+    rng = np.random.default_rng(3)
+    cases = 0
+    for tag in ('qubit', 'transmon', 'coupled'):
+        L, dt = list(unit_golden['disc_%s_L' % tag]), float(unit_golden['disc_%s_dt' % tag])
+        c, m = L[0].shape[0], len(L) - 1
+        for order in (1, 2, 3):
+            key = 'disc_%s_o%d' % (tag, order)
+            if key not in unit_golden:
+                continue
+            blocks = unit_golden[key].reshape(c, -1, c).transpose(1, 0, 2)
+            found = _reference_monomial_order(L, dt, order, blocks, rng)
+            assert found == rs.power_table(order, m).tolist(), (tag, order)
+            assert found == [list(p) for p in linearize.create_power_list(order, m)], (tag, order)
+            cases += 1
+    assert cases == 8
+    if refshim.available():
+        lin = refshim.module('linearize')
+        for order, m in ((2, 2), (3, 1), (3, 3)):
+            assert [list(p) for p in lin.create_power_list(order, m)] == rs.power_table(order, m).tolist()
 
 
 def test_process_maps_and_gate_loop_vs_reference():

@@ -27,11 +27,11 @@ __host__ __device__ constexpr int cmax(int a, int b) { return a > b ? a : b; }
 
 // ---------------------------------------------------------------------------------------------------------
 // Compile-time configuration for a (complex state dim, control dim) pair.
-// The two dense products of a Riccati stage, W = P G and T = G^T W with G = [A_t | B_t] (N x Q), run on the fp64
-// tensor cores (mma.sync m8n8k4, "DMMA"): operands padded to NP = rup(N, 8) rows, QP = rup(Q, 8) columns and
-// KP = rup(N, 4) in the contraction; leading dimensions chosen so that the fragment loads are free of bank
-// conflicts: a 64-bit warp load is served per half warp (fragment rows 0..3 x columns 0..3), which wants the row
-// stride to be 4 or 12 mod 16 doubles for both the A-type (row = lane/4) and the B-type (row = lane%4) pattern.
+// The two dense products of a Riccati stage run on the fp64 tensor cores (mma.sync m8n8k4, "DMMA"):
+// W^T = G^T P stays in the DMMA accumulators and feeds the second product T = W^T G straight from registers.  That
+// works without a single shuffle because the contraction index of a k-step is free to be permuted: step (kt, e)
+// contracts over k = 8 kt + 2 c4 + e, which is exactly the column the accumulator fragment of lane (g8, c4) holds.
+// Operand rows are then 2 LD apart between neighbouring c4, so conflict-free fragment loads want LD = 2 or 6 (mod 8).
 // MAXW: most warps (members) a CTA is ever launched with; it fixes the register budget (__launch_bounds__).
 // ---------------------------------------------------------------------------------------------------------
 __host__ __device__ constexpr int next_mod(int x, int r, int m) { return x + ((r - x % m) % m + m) % m; }
@@ -52,24 +52,12 @@ template <> struct Tiles<16, 1> { static constexpr int MAXW = 8; };
 template <int C_, int M_> struct Cfg {
     static constexpr int C = C_, N = 2 * C_, M = M_, Q = N + M_;
     static constexpr int MAXW = Tiles<C_, M_>::MAXW;
-    static constexpr int NP = rup(N, 8), QP = rup(Q, 8), KP = rup(N, 4);
-    static constexpr int MT = NP / 8, QT = QP / 8, KS = KP / 4;   // tile counts
-    static constexpr int LDP = cmin(next_mod(KP, 4, 16), next_mod(KP, 12, 16));
-    static constexpr int LDG = cmin(next_mod(QP, 4, 16), next_mod(QP, 12, 16));
-    static_assert(LDP >= Q && LDP % 2 == 0, "T11 and the control columns are staged in the P buffer");
-    static_assert(QP > Q, "one padding column of G carries the affine term");
-    // Second-generation factor (riccati_factor2, N <= 24): W^T = G^T P stays in the DMMA accumulators and feeds the
-    // second product T = W^T G straight from registers.  That works without a single shuffle because the contraction
-    // index of a k-step is free to be permuted: step (kt, e) contracts over k = 8 kt + 2 c4 + e, which is exactly the
-    // column the accumulator fragment of lane (g8, c4) holds.  Operand rows are then 2 LD apart between neighbouring
-    // c4, so conflict-free fragment loads want LD = 2 or 6 (mod 8).
-    static constexpr int NT = cdiv(N, 8), GT = cdiv(Q + 1, 8), TT = cdiv(Q, 8);
+    static constexpr int NT = cdiv(N, 8), GT = cdiv(Q + 1, 8), TT = cdiv(Q, 8);   // tile counts
     // operand rows: the N real ones plus, when N is not a multiple of 8, ONE row of zeros that every padding index of
     // the last contraction tile is mapped to (instead of 8 NT - N zero rows: 2 x 130 doubles less per member for N = 18)
     static constexpr int KR = (N % 8 == 0) ? N : N + 1;
-    static constexpr bool FAC2 = NT <= 3;
-    static constexpr int LDP2 = cmin(next_mod(8 * NT, 2, 8), next_mod(8 * NT, 6, 8));
-    static constexpr int LDG2 = cmin(next_mod(8 * GT, 2, 8), next_mod(8 * GT, 6, 8));
+    static constexpr int LDP = cmin(next_mod(8 * NT, 2, 8), next_mod(8 * NT, 6, 8));
+    static constexpr int LDG = cmin(next_mod(8 * GT, 2, 8), next_mod(8 * GT, 6, 8));
 };
 
 // ---------------------------------------------------------------------------------------------------------
@@ -105,16 +93,15 @@ template <class CF> struct Rec {
     static_assert(B % 2 == 0 && SMALL % 2 == 0 && SIZE % 2 == 0, "records are moved in 16-byte chunks");
     // offset of K[a][k] / B[k][i] (k = realified state index) inside their pair blocks
     __host__ __device__ static constexpr int pair(int ctl, int k) { return (ctl * CF::C + (k % CF::C)) * 2 + (k >= CF::C); }
-    // during the vector sweeps whole records are staged in the [G | W] buffers (only live inside the factor)
-    static_assert(CF::FAC2 ? SLOT + SIZE <= CF::KR * (CF::LDP2 + CF::LDG2) : SLOT + SIZE <= (CF::KP + CF::NP) * CF::LDG,
-                  "record ring does not fit the factor scratch");
+    // during the vector sweeps whole records are staged in the [P | G] buffers (only live inside the factor)
+    static_assert(SLOT + SIZE <= CF::KR * (CF::LDP + CF::LDG), "record ring does not fit the factor scratch");
 };
 template <class CF> __host__ __device__ constexpr int ws_doubles(int H) {
     return H * Rec<CF>::SIZE + 2 * (H + 1) * CF::N;
 }
 
 template <class CF> struct Slab {
-    double *P, *AB, *W, *T21, *S, *ring, *kk, *hl, *Ug, *Uo, *z, *y, *x0, *va, *vb, *xT, *lo0, *hi0, *xcur, *xmeas, *scr, *mbar;
+    double *P, *AB, *W, *T21, *S, *ring, *kk, *hl, *Ug, *Uo, *z, *y, *x0, *va, *vb, *xT, *lo0, *hi0, *xcur, *xmeas, *scr;
     double *recring;   // 2-slot ring of whole stage records for the vector sweeps (aliases the factor scratch)
     double *xd;        // 2 N doubles of scratch for the general-cost adjoint sweep
     int *mask;
@@ -124,8 +111,8 @@ template <class CF> struct Slab {
         return layout(nullptr, nullptr, H, nblk, dd);
     }
     // scratch of the linearisation (2 x [p][M] derivative weights) and of the plant step (4 complex d x d):
-    // aliases W, which is only live inside the Riccati factor
-    __host__ __device__ static constexpr int scratch_doubles() { return CF::FAC2 ? CF::KR * CF::LDG2 : CF::NP * CF::LDG; }
+    // aliases G, which is only live inside the Riccati factor
+    __host__ __device__ static constexpr int scratch_doubles() { return CF::KR * CF::LDG; }
     __host__ __device__ static bool scratch_fits(int nblk, int dd) {
         return cmax(8 * dd, 2 * CF::M * nblk) <= scratch_doubles();
     }
@@ -140,19 +127,11 @@ template <class CF> struct Slab {
         };
         Slab dummy;
         Slab *q = s ? s : &dummy;
-        if (CF::FAC2) {
-            take(&q->P, CF::KR * CF::LDP2, 16);   // P_{t+1}, zero padded, [KR][LDP2]
-            take(&q->AB, CF::KR * CF::LDG2);  // G = [A_t | B~_t | D~_t], zero padded, [KR][LDG2]
-            take(&q->W, M * N);               // K_t for the update of P (W = P G itself never leaves the registers)
-            q->scr = q->AB;
-            q->recring = q->P;
-        } else {
-            take(&q->P, CF::NP * CF::LDP);    // P_{t+1}, zero padded
-            take(&q->AB, CF::KP * CF::LDG, 16);   // G = [A_t | B~_t], zero padded
-            take(&q->W, CF::NP * CF::LDG);    // W = P G
-            q->scr = q->W;
-            q->recring = q->AB;
-        }
+        take(&q->P, CF::KR * CF::LDP, 16);   // P_{t+1}, zero padded, [KR][LDP]
+        take(&q->AB, CF::KR * CF::LDG);      // G = [A_t | B~_t | D~_t], zero padded, [KR][LDG]
+        take(&q->W, M * N);                  // K_t for the update of P (W = P G itself never leaves the registers)
+        q->scr = q->AB;
+        q->recring = q->P;
         take(&q->xd, 2 * N);
         take(&q->T21, M * N);
         take(&q->S, M * M);
@@ -167,7 +146,6 @@ template <class CF> struct Slab {
         take(&q->va, N + 2);   // sweep vectors: imaginary half at offset rup(C, 2)
         take(&q->vb, N + 2);
         take(&q->xT, N);
-        take(&q->mbar, 4);   // two mbarriers (one per record-ring slot) + their phase bits
         take(&q->lo0, M);
         take(&q->hi0, M);
         take(&q->xcur, 2 * dd);
@@ -225,51 +203,6 @@ template <int COUNT> __device__ __forceinline__ void prefetch_block(double *dst,
     for (int c = 0; c < cdiv(COUNT / 2, 32); ++c, sa += 512, ga += 512)
         if (c * 32 + lane < COUNT / 2) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(ga) : "memory");
     cp_async_commit();
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Record ring of the vector sweeps, optional TMA variant (compile with -DM4Q_TMA_RING=1): whole stage records
-// (2.3 KB for the transmon) moved as 1-D bulk copies (cp.async.bulk, UBLKCP in SASS), one instruction of one lane per
-// record, completion on an mbarrier per ring slot.  The records are written through the generic proxy (plain stores of
-// this warp) and read by the bulk copy through the async proxy, so a proxy fence precedes every issue.  Measured on
-// B200 (transmon_h16, 65,536 members): LDGSTS ring 116.2 k trajectories/s; bulk copies with fence.proxy.async.global
-// 115.0 k, with the full fence.proxy.async 101.4 k -- no gain at this transfer size, so LDGSTS stays the default.
-// ---------------------------------------------------------------------------------------------------------
-#ifndef M4Q_TMA_RING
-#define M4Q_TMA_RING 0
-#endif
-#ifndef M4Q_PROXY_FENCE
-#define M4Q_PROXY_FENCE "fence.proxy.async.global;"
-#endif
-__device__ __forceinline__ void mbar_init(double *mbar, int lane) {
-    if (lane == 0) {
-        const unsigned a = (unsigned)__cvta_generic_to_shared(mbar);
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(a) : "memory");
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(a + 8) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        reinterpret_cast<unsigned *>(mbar + 2)[0] = 0u;   // phase bits of the two slots
-    }
-    __syncwarp();
-}
-__device__ __forceinline__ void bulk_load(double *dst, const double *src, unsigned bytes, double *mbar_slot) {
-    const unsigned d = (unsigned)__cvta_generic_to_shared(dst), m = (unsigned)__cvta_generic_to_shared(mbar_slot);
-    asm volatile(M4Q_PROXY_FENCE ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(m), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(d),
-                 "l"(__cvta_generic_to_global(src)), "r"(bytes), "r"(m)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(double *mbar_slot, unsigned parity) {
-    const unsigned m = (unsigned)__cvta_generic_to_shared(mbar_slot);
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@!p bra WAIT_%=;\n"
-        "}\n" ::"r"(m),
-        "r"(parity)
-        : "memory");
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -521,277 +454,8 @@ template <class CF> __device__ __forceinline__ double box_hi(const Slab<CF> &s, 
 // ---------------------------------------------------------------------------------------------------------
 // Riccati matrix sweep.  masked: controls with mask != 0 are pinned to their bound (polish), rho_half = 0.
 // Produces K_t, S_t^-1, dv_t = P_{t+1} (D_t + B_fixed b) for all stages (written to the stage records).
-//
-// Per stage, with G = [A_t | B~_t] (N x Q):  W = P G, then T = G^T W, both as DMMA tile products with the
-// accumulators in registers.  T is symmetric: only its upper block triangle is computed; the lanes that hold the
-// control columns publish T12 (= T21^T) and T22, and after one warp sync the update
-//   P_t = Qbar_t + T11 - T21^T S^-1 T21,   S = R + rho/2 + T22
-// is applied to the accumulator fragments and mirrored, so P stays exactly symmetric and T11 never touches memory.
-// ---------------------------------------------------------------------------------------------------------
-template <class CF, bool FUSED>
-__device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, const QPData &qp_in, double rho_half,
-                                            bool masked, int lane) {
-    constexpr int C = CF::C, N = CF::N, M = CF::M, Q = CF::Q;
-    constexpr int NP = CF::NP, KP = CF::KP, LDP = CF::LDP, LDG = CF::LDG, MT = CF::MT, QT = CF::QT, KS = CF::KS;
-    using R_ = Rec<CF>;
-    const Slab<CF> s = slab_view<CF>(sr);
-    const StageOps ops = localize<FUSED>(ops_in);
-    const QPData qp = localize<FUSED>(qp_in);
-    const int H = sr.H;
-    const int g8 = lane >> 2, c4 = lane & 3;   // fragment coordinates of this lane
-    // the pairs (i <= j) of the symmetric P update this lane owns, fixed for the whole sweep: packed (i << 8) | j
-    constexpr int NTRI = N * (N + 1) / 2, NPAIR = cdiv(NTRI, 32);
-    int pair[NPAIR];
-    {
-        int i = 0, j = lane;   // element `lane` of the row-major upper triangle, then every 32nd
-        while (i < N && j >= N) {
-            j += i + 1 - N;
-            ++i;
-        }
-#pragma unroll
-        for (int q = 0; q < NPAIR; ++q) {
-            pair[q] = (i < N) ? ((i << 8) | j) : -1;
-            j += 32;
-            while (i < N && j >= N) {
-                j += i + 1 - N;
-                ++i;
-            }
-        }
-    }
-    // P <- Qf with zero padding; G, W padding rows / columns zeroed once (never written afterwards)
-#pragma unroll 1
-    for (int e = lane; e < NP * LDP; e += 32) {
-        const int i = e / LDP, j = e % LDP;
-        s.P[e] = (i < N && j < N) ? qp.Qf[i * N + j] : 0.0;
-    }
-#pragma unroll 1
-    for (int e = lane; e < KP * LDG; e += 32) s.AB[e] = 0.0;
-    constexpr int BD = R_::SMALL - R_::B;   // [B_t | D_t]
-    prefetch_block<BD>(s.ring + ((H - 1) & 1) * R_::BDSLOT, ws_rec<CF>(sr, H - 1) + R_::B, lane);
-#pragma unroll 1
-    for (int t = H - 1; t >= 0; --t) {
-        const double *ug_t = s.Ug + t * M;
-        const double2 *blk0 = ops.blocks + (size_t)t * ops.stage_stride;
-        const double *Bt = s.ring + (t & 1) * R_::BDSLOT, *Dt = Bt + (R_::D - R_::B);
-        double *rec = ws_rec<CF>(sr, t);
-        cp_async_wait_all();
-        __syncwarp();   // B_t, D_t have landed; P_{t+1} of the previous stage is complete
-        if (t > 0) prefetch_block<BD>(s.ring + ((t - 1) & 1) * R_::BDSLOT, ws_rec<CF>(sr, t - 1) + R_::B, lane);
-        // realified A_t = sum_k phi_k block_k into G[:, 0:N] (and, complex, into the record for the vector sweeps)
-        {
-            constexpr int NE = cdiv(C * C, 32);
-            double ar[NE], ai[NE];
-#pragma unroll
-            for (int q = 0; q < NE; ++q) ar[q] = ai[q] = 0.0;
-            const double2 *bp = blk0 + lane;
-            // loads of one block issued together (NE independent 16-byte loads), clamped instead of predicated
-            const int qlast = (C * C - 1 - lane) >> 5;   // last valid q of this lane
-#pragma unroll 1
-            for (int kb = 0; kb < ops.nblk; ++kb, bp += C * C) {
-                const double ph = stage_weight<M>(ops, ug_t, kb);
-                double2 v[NE];
-#pragma unroll
-                for (int q = 0; q < NE; ++q) v[q] = bp[32 * (q < qlast ? q : qlast)];
-#pragma unroll
-                for (int q = 0; q < NE; ++q) {
-                    ar[q] = fma(ph, v[q].x, ar[q]);
-                    ai[q] = fma(ph, v[q].y, ai[q]);
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < NE; ++q) {
-                const int e = lane + 32 * q;
-                if (e < C * C) {
-                    const int r = e / C, j = e % C;
-                    s.AB[r * LDG + j] = ar[q];
-                    s.AB[r * LDG + C + j] = -ai[q];
-                    s.AB[(C + r) * LDG + j] = ai[q];
-                    s.AB[(C + r) * LDG + C + j] = ar[q];
-                    reinterpret_cast<double2 *>(rec + R_::AT)[r * R_::CA + j] = make_double2(ar[q], ai[q]);
-                }
-            }
-        }
-        // B~ into G[:, N:Q]
-#pragma unroll 1
-        for (int e = lane; e < N * M; e += 32) {
-            const int k = e / M, i = e % M;
-            const bool fixed = masked && s.mask[t * M + i] != 0;
-            s.AB[k * LDG + N + i] = fixed ? 0.0 : Bt[R_::pair(i, k)];
-        }
-        if (lane < N) {   // D~ rides along as column Q of G: W[:, Q] = P_{t+1} D~ = dv_t comes out of the first product
-            double dt = Dt[lane];
-            if (masked) {
-#pragma unroll
-                for (int i = 0; i < M; ++i) {
-                    const int mk = s.mask[t * M + i];
-                    if (mk) dt = fma(Bt[R_::pair(i, lane)], mk == 1 ? box_lo(s, qp.sat, t, i) : box_hi(s, qp.sat, t, i), dt);
-                }
-            }
-            s.AB[lane * LDG + Q] = dt;
-        }
-        __syncwarp();
-        // ---- W = P G : MT x QT tiles, KS k-steps (rolled: the hot code has to fit the instruction cache)
-        {
-            double w[MT][QT][2];
-#pragma unroll
-            for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) w[mi][ni][0] = w[mi][ni][1] = 0.0;
-            const double *pa = s.P + g8 * LDP + c4;      // A fragment: P[mi*8 + g8][ks*4 + c4]
-            const double *gb = s.AB + c4 * LDG + g8;     // B fragment: G[ks*4 + c4][ni*8 + g8]
-            // software pipelined: the fragments of k-step ks + 1 are in flight while the MMAs of ks issue
-            double af[MT], bf[QT];
-#pragma unroll
-            for (int mi = 0; mi < MT; ++mi) af[mi] = pa[mi * 8 * LDP];
-#pragma unroll
-            for (int ni = 0; ni < QT; ++ni) bf[ni] = gb[ni * 8];
-#pragma unroll 1
-            for (int ks = 0; ks < KS; ++ks) {
-                double an[MT], bn[QT];
-                const int adv = ks + 1 < KS ? 1 : 0;   // the last step re-loads its own fragments (no branch)
-                pa += 4 * adv;
-                gb += 4 * LDG * adv;
-#pragma unroll
-                for (int mi = 0; mi < MT; ++mi) an[mi] = pa[mi * 8 * LDP];
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) bn[ni] = gb[ni * 8];
-#pragma unroll
-                for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-                    for (int ni = 0; ni < QT; ++ni) dmma(w[mi][ni], af[mi], bf[ni]);
-#pragma unroll
-                for (int mi = 0; mi < MT; ++mi) af[mi] = an[mi];
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) bf[ni] = bn[ni];
-            }
-            double2 *wd = reinterpret_cast<double2 *>(s.W + g8 * LDG + 2 * c4);
-#pragma unroll
-            for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) wd[(mi * 8 * LDG + ni * 8) >> 1] = make_double2(w[mi][ni][0], w[mi][ni][1]);
-        }
-        __syncwarp();
-        if (lane < N) rec[R_::DV + lane] = s.W[lane * LDG + Q];
-        // ---- T = G^T W, upper block triangle: tile (mi <= ni) holds T[mi*8 + g8][ni*8 + 2*c4 + {0,1}].
-        // T11 goes into the P buffer (P_{t+1} is dead: it was the A operand of the first product), the control
-        // columns T12 = T21^T and T22 into their own small arrays.
-        {
-            double tt[QT][QT][2];
-#pragma unroll
-            for (int mi = 0; mi < QT; ++mi)
-#pragma unroll
-                for (int ni = mi; ni < QT; ++ni) tt[mi][ni][0] = tt[mi][ni][1] = 0.0;
-            const double *ga = s.AB + c4 * LDG + g8;     // A fragment: G^T[mi*8 + g8][ks*4 + c4] = G[ks*4 + c4][mi*8 + g8]
-            const double *wb = s.W + c4 * LDG + g8;      // B fragment: W[ks*4 + c4][ni*8 + g8]
-            double af[QT], bf[QT];
-#pragma unroll
-            for (int mi = 0; mi < QT; ++mi) af[mi] = ga[mi * 8];
-#pragma unroll
-            for (int ni = 0; ni < QT; ++ni) bf[ni] = wb[ni * 8];
-#pragma unroll 1
-            for (int ks = 0; ks < KS; ++ks) {
-                double an[QT], bn[QT];
-                const int adv = ks + 1 < KS ? 4 * LDG : 0;
-                ga += adv;
-                wb += adv;
-#pragma unroll
-                for (int mi = 0; mi < QT; ++mi) an[mi] = ga[mi * 8];
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) bn[ni] = wb[ni * 8];
-#pragma unroll
-                for (int mi = 0; mi < QT; ++mi)
-#pragma unroll
-                    for (int ni = mi; ni < QT; ++ni) dmma(tt[mi][ni], af[mi], bf[ni]);
-#pragma unroll
-                for (int mi = 0; mi < QT; ++mi) af[mi] = an[mi];
-#pragma unroll
-                for (int ni = 0; ni < QT; ++ni) bf[ni] = bn[ni];
-            }
-            // publish, branch free: elements outside T11 / T12 / T22 go to a dummy slot (va is unused in the factor)
-#pragma unroll
-            for (int mi = 0; mi < QT; ++mi)
-#pragma unroll
-                for (int ni = mi; ni < QT; ++ni) {
-                    const int i = mi * 8 + g8, j = ni * 8 + 2 * c4;   // N and j even: the pair (j, j+1) is on one side
-                    if (ni * 8 + 7 < N) {          // whole tile left of the control columns (compile time)
-                        double *dst = (mi * 8 + 7 < N || i < N) ? s.P + i * LDP + j : s.va;
-                        *reinterpret_cast<double2 *>(dst) = make_double2(tt[mi][ni][0], tt[mi][ni][1]);
-                    } else {
-                        if (ni * 8 < N) {          // tile straddles: its left pairs still belong to T11
-                            double *dst = (j < N && i < N) ? s.P + i * LDP + j : s.va;
-                            *reinterpret_cast<double2 *>(dst) = make_double2(tt[mi][ni][0], tt[mi][ni][1]);
-                        }
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const int jj = j + e;
-                            const bool ctl = jj >= N && jj < Q;
-                            double *d1 = (ctl && i < N) ? s.T21 + (jj - N) * N + i : s.va + 2;
-                            *d1 = tt[mi][ni][e];
-                            if (mi == ni || (mi * 8 + 7 >= N)) {   // rows that can reach into T22 (compile time)
-                                const bool s22 = ctl && i >= N && i <= jj;
-                                double *d2 = s22 ? s.S + (i - N) * M + (jj - N) : s.va + 3;
-                                double *d3 = s22 ? s.S + (jj - N) * M + (i - N) : s.va + 3;
-                                *d2 = tt[mi][ni][e];
-                                *d3 = tt[mi][ni][e];
-                            }
-                        }
-                    }
-                }
-        }
-        __syncwarp();
-        // S = R~ + rho/2 + B~^T P B~ ; invert (every lane redundantly, M <= 3)
-        double Sm[M][M], Si[M][M];
-        const double *Rt = qp.R + t * qp.r_stride;
-#pragma unroll
-        for (int a = 0; a < M; ++a) {
-            const bool fa = masked && s.mask[t * M + a] != 0;
-#pragma unroll
-            for (int b = 0; b < M; ++b) {
-                const bool fb = masked && s.mask[t * M + b] != 0;
-                double v = s.S[a * M + b];
-                if (fa || fb) v = (a == b) ? 1.0 : 0.0;
-                else v += Rt[a * M + b] + (a == b ? rho_half : 0.0);
-                Sm[a][b] = v;
-            }
-        }
-        spd_inverse<M>(Sm, Si);
-        if (lane == 0) {
-#pragma unroll
-            for (int a = 0; a < M; ++a)
-#pragma unroll
-                for (int b = 0; b < M; ++b) rec[R_::SINV + a * M + b] = Si[a][b];
-        }
-        if (lane < N) {
-#pragma unroll
-            for (int a = 0; a < M; ++a) {
-                double kv = 0.0;
-#pragma unroll
-                for (int b = 0; b < M; ++b) kv = fma(Si[a][b], s.T21[b * N + lane], kv);
-                rec[R_::K + R_::pair(a, lane)] = kv;
-                s.W[a * N + lane] = kv;   // W is dead after the second product
-            }
-        }
-        __syncwarp();
-        // P_t = Qbar_t + T11 - T21^T K, in place on the upper triangle and mirrored
-        const double *Qt = qp.Q + t * qp.q_stride;
-#pragma unroll
-        for (int q = 0; q < NPAIR; ++q) {
-            if (pair[q] < 0) continue;
-            const int i = pair[q] >> 8, j = pair[q] & 255;
-            double v = s.P[i * LDP + j];
-            if (!qp.q_diag || i == j) v += Qt[i * N + j];
-#pragma unroll
-            for (int a = 0; a < M; ++a) v = fma(-s.T21[a * N + i], s.W[a * N + j], v);
-            s.P[i * LDP + j] = v;
-            s.P[j * LDP + i] = v;
-        }
-    }
-    __syncwarp();
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Second-generation Riccati matrix sweep (CF::FAC2).  Same mathematics and the same outputs as riccati_factor;
-// what changes is the traffic through shared memory, the resource this kernel is bound by:
+// Per stage  T = G^T P_{t+1} G,  S = R + rho/2 + T22,  P_t = Qbar_t + T11 - T21^T S^-1 T21.  Shared memory is the
+// resource this kernel is bound by, so the products keep their traffic through it small:
 //   * W^T = G^T P (G = [A_t | B~_t | D~_t], N x (Q + 1)) is accumulated in DMMA fragments and consumed by the second
 //     product T = W^T G straight from the registers: a k-step (kt, e) contracts over k = 8 kt + 2 c4 + e, the very
 //     column of W^T that lane (g8, c4) holds in accumulator element e, so the A operand of the second product IS
@@ -803,10 +467,10 @@ __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, 
 //     upper block triangle and its mirror image, so P stays exactly symmetric.
 // ---------------------------------------------------------------------------------------------------------
 template <class CF, bool FUSED>
-__device__ __noinline__ void riccati_factor2(SlabRef sr, const StageOps &ops_in, const QPData &qp_in, double rho_half,
-                                             bool masked, int lane) {
+__device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, const QPData &qp_in, double rho_half,
+                                            bool masked, int lane) {
     constexpr int C = CF::C, N = CF::N, M = CF::M, Q = CF::Q;
-    constexpr int NT = CF::NT, GT = CF::GT, TT = CF::TT, KR = CF::KR, LDP = CF::LDP2, LDG = CF::LDG2;
+    constexpr int NT = CF::NT, GT = CF::GT, TT = CF::TT, KR = CF::KR, LDP = CF::LDP, LDG = CF::LDG;
     constexpr bool LASTNAT = (N % 8 != 0) && (N % 8 <= 4);   // ragged last contraction tile: one k-step of 4 indices
     constexpr int KSTEPS = 2 * NT - (LASTNAT ? 1 : 0);
     using R_ = Rec<CF>;
@@ -1082,39 +746,13 @@ __device__ __noinline__ void riccati_factor2(SlabRef sr, const StageOps &ops_in,
     __syncwarp();
 }
 
-template <class CF, bool FUSED>
-__device__ __forceinline__ void factor_dispatch(const SlabRef &sr, const StageOps &ops, const QPData &qp, double rho_half,
-                                                bool masked, int lane) {
-    if constexpr (CF::FAC2) riccati_factor2<CF, FUSED>(sr, ops, qp, rho_half, masked, lane);
-    else riccati_factor<CF, FUSED>(sr, ops, qp, rho_half, masked, lane);
-}
-
-// stage record t of the workspace -> slot (t & 1) of the record ring in the [G | W] buffers
+// stage record t of the workspace -> slot (t & 1) of the record ring in the [P | G] buffers
 template <class CF> __device__ __forceinline__ double *rec_slot(const Slab<CF> &s, int t) {
     return s.recring + (t & 1) * Rec<CF>::SLOT;
 }
 template <class CF>
 __device__ __forceinline__ void prefetch_stage(const Slab<CF> &s, const SlabRef &sr, int t, int lane) {
-#if M4Q_TMA_RING
-    if (lane == 0) bulk_load(rec_slot<CF>(s, t), ws_rec<CF>(sr, t), Rec<CF>::SIZE * 8, s.mbar + (t & 1));
-#else
     prefetch_block<Rec<CF>::SIZE>(rec_slot<CF>(s, t), ws_rec<CF>(sr, t), lane);
-#endif
-}
-// wait for record t; ph carries the phase bits of the two slots (uniform over the warp, kept in the slab between calls)
-template <class CF> __device__ __forceinline__ void ring_wait(const Slab<CF> &s, int t, unsigned &ph) {
-#if M4Q_TMA_RING
-    mbar_wait(s.mbar + (t & 1), (ph >> (t & 1)) & 1u);
-    ph ^= 1u << (t & 1);
-#else
-    cp_async_wait_all();
-#endif
-}
-template <class CF> __device__ __forceinline__ unsigned ring_phase_load(const Slab<CF> &s) {
-    return reinterpret_cast<const unsigned *>(s.mbar + 2)[0];
-}
-template <class CF> __device__ __forceinline__ void ring_phase_store(const Slab<CF> &s, unsigned ph, int lane) {
-    if (lane == 0) reinterpret_cast<unsigned *>(s.mbar + 2)[0] = ph;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1147,7 +785,6 @@ __device__ __noinline__ double riccati_solve(SlabRef sr, const QPData &qp_in, do
     // the refinement variant is a separate (cold) instantiation: the hot copy stays small for the instruction cache
     const bool adj = !REFINE && mode == SWEEP_ADJOINT, refine = REFINE;
     double *Xo = ws_Xo<CF>(sr);
-    unsigned ph = ring_phase_load<CF>(s);
     prefetch_stage<CF>(s, sr, H - 1, lane);
 #pragma unroll 1
     for (int e = lane; e < H * M; e += 32) {
@@ -1203,7 +840,7 @@ __device__ __noinline__ double riccati_solve(SlabRef sr, const QPData &qp_in, do
             dv_n = ws_rec<CF>(sr, t - 1)[R_::DV + lane];
             ql_n = qp.qlin[(t - 1) * N + lane];
         }
-        ring_wait<CF>(s, t, ph);
+        cp_async_wait_all();
         __syncwarp();
         if (t > 0) prefetch_stage<CF>(s, sr, t - 1, lane);
         if (adj && act) ql = -2.0 * qp.Q[t * qp.q_stride + lane * N + lane] * slot[R_::XC + lane];
@@ -1244,7 +881,6 @@ __device__ __noinline__ double riccati_solve(SlabRef sr, const QPData &qp_in, do
     }
     __syncwarp();   // kk complete; va/vb free again
     if (adj) {      // max |grad| over the horizon
-        ring_phase_store<CF>(s, ph, lane);
         double gm = 0.0;
 #pragma unroll 1
         for (int e = lane; e < H * M; e += 32) gm = fmax(gm, fabs(s.kk[e]));
@@ -1269,7 +905,7 @@ __device__ __noinline__ double riccati_solve(SlabRef sr, const QPData &qp_in, do
                 r_n = qp.r[(t + 1) * N + lane];
             }
         }
-        if (t > 0) ring_wait<CF>(s, t, ph);   // record 0 is still in its slot from the backward sweep
+        if (t > 0) cp_async_wait_all();   // record 0 is still in its slot from the backward sweep
         __syncwarp();
         if (t + 1 < H) prefetch_stage<CF>(s, sr, t + 1, lane);
         int mk[M];
@@ -1311,7 +947,6 @@ __device__ __noinline__ double riccati_solve(SlabRef sr, const QPData &qp_in, do
         }
     }
     if (act) s.xT[lane] = refine ? s.xT[lane] + x : x - (WRITE_X ? r_n : qp.r[H * N + lane]);
-    ring_phase_store<CF>(s, ph, lane);
     __syncwarp();
     // a non-finite state anywhere in the rollout propagates to x_H
     const bool bad = __any_sync(FULL, !isfinite(x));
@@ -1349,7 +984,6 @@ __device__ __noinline__ double adjoint_gradient(SlabRef sr, const QPData &qp_in,
     const int H = sr.H;
     const bool act = lane < N;
     const double *Xo = ws_Xo<CF>(sr);
-    unsigned ph = ring_phase_load<CF>(s);
     prefetch_stage<CF>(s, sr, H - 1, lane);
     double xd_n = act ? Xo[(H - 1) * N + lane] - qp.r[(H - 1) * N + lane] : 0.0;
     if (act) s.xd[lane] = Xo[H * N + lane] - qp.r[H * N + lane];
@@ -1370,7 +1004,7 @@ __device__ __noinline__ double adjoint_gradient(SlabRef sr, const QPData &qp_in,
             xdv[lane] = xd;
             if (t > 0) xd_n = Xo[(t - 1) * N + lane] - qp.r[(t - 1) * N + lane];
         }
-        ring_wait<CF>(s, t, ph);
+        cp_async_wait_all();
         __syncwarp();
         if (t > 0) prefetch_stage<CF>(s, sr, t - 1, lane);
         double g[M];
@@ -1390,7 +1024,6 @@ __device__ __noinline__ double adjoint_gradient(SlabRef sr, const QPData &qp_in,
         const double atl = cmatvec<CF, true, R_::CA>(At, lamv, lane);
         lam = atl + 2.0 * apply_Q<CF>(qp.Q + t * qp.q_stride, qp.q_diag, xdv, lane);
     }
-    ring_phase_store<CF>(s, ph, lane);
     __syncwarp();
     return gmax;
 }
@@ -1415,7 +1048,7 @@ __device__ __noinline__ void admm_block(SlabRef sr, const StageOps &ops_in, cons
             // is rescaled by sqrt(normalised primal residual / normalised dual residual) when that ratio is far from
             // one, the scaled dual y follows, and the Riccati factorisation is redone with the new rho.
             double rho = set.rho, rh = rho_half;
-            factor_dispatch<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
+            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
             cnt.factor++;
             int next_check = 5;
             for (int it = 0; it < set.max_admm; ++it) {
@@ -1458,7 +1091,7 @@ __device__ __noinline__ void admm_block(SlabRef sr, const StageOps &ops_in, cons
                         __syncwarp();
                         rho = rho_new;
                         rh = 0.5 * rho;
-                        factor_dispatch<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
+                        riccati_factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
                         cnt.factor++;
                     }
                 }
@@ -1517,7 +1150,7 @@ __device__ int qp_solve(SlabRef sr, const StageOps &ops_in, const QPData &qp_in,
         if (kkt_ok && ((set.kkt_mode >= 2 && cnt.sticky) || set.kkt_mode >= 4)) {
             // an earlier QP of this member needed the pivoted KKT solve (cost-to-go beyond fp64: order-1 model at long
             // horizons): go straight to it.  One factor call forms the stage operators A_t in the records.
-            factor_dispatch<CF, FUSED>(sr, ops_in, qp_in, 0.0, false, lane);
+            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, 0.0, false, lane);
             status = kkt_active_set<CF, FUSED>(sr, qp_in, set, lane, cnt);
             break;
         }
@@ -1564,7 +1197,7 @@ __device__ int qp_solve(SlabRef sr, const StageOps &ops_in, const QPData &qp_in,
         bool certified = false;
         bool numeric = false;   // the rounds ended on a settled working set whose solve is not stationary, or not finite
         for (int round = 0; round < set.max_polish; ++round) {
-            factor_dispatch<CF, FUSED>(sr, ops_in, qp_in, 0.0, true, lane);
+            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, 0.0, true, lane);
             cnt.factor++;
             cnt.polish++;
             x_nonfinite = riccati_solve<CF, FUSED>(sr, qp_in, 0.0, SWEEP_POLISH, true, lane) != 0.0;

@@ -353,8 +353,7 @@ template <class CF>
 __device__ __noinline__ void linearize_exact(SlabRef sr, const double2 *gen, double dt, double2 *At, int lane) {
     constexpr int C = CF::C, N = CF::N, M = CF::M, CC = C * C;
     using R_ = Rec<CF>;
-    static_assert(2 * exact_scratch<CF>() <= (CF::FAC2 ? CF::KR * (CF::LDP2 + CF::LDG2) : (CF::KP + CF::NP) * CF::LDG),
-                  "exact-stage scratch must fit the factor scratch");
+    static_assert(2 * exact_scratch<CF>() <= CF::KR * (CF::LDP + CF::LDG), "exact-stage scratch must fit the factor scratch");
     const Slab<CF> s = slab_view<CF>(sr);
     const double *Xg = ws_Xg<CF>(sr);
     double2 *scr = reinterpret_cast<double2 *>(s.recring);
@@ -428,7 +427,6 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
     const Slab<CF> s = slab_view<CF>(sr);
     double *Xg = ws_Xg<CF>(sr);
     const double *Xo = ws_Xo<CF>(sr);
-    mbar_init(s.mbar, lane);
     double2 *xcur = reinterpret_cast<double2 *>(s.xcur);
     double2 *xmeas = reinterpret_cast<double2 *>(s.xmeas);
     double2 *scr2 = reinterpret_cast<double2 *>(s.scr);
@@ -807,7 +805,6 @@ __global__ void __launch_bounds__(CF::MAXW * 32) qp_kernel(const QpArgs a) {
     const int H = a.H;
     SlabRef sr = {warp * a.slab_doubles, H, 1, C, nullptr};
     const Slab<CF> s = slab_view<CF>(sr);
-    mbar_init(s.mbar, lane);
 
     for (long long k = (long long)blockIdx.x * wpc + warp; k < a.n_inst; k += (long long)gridDim.x * wpc) {
         double *ws = a.ws + k * qp_ws_doubles<CF>(H);

@@ -251,11 +251,12 @@ def _random_qp(rng, c, m, H, hermitian_cost, with_du):
     U_bm = 0.3 * rng.standard_normal((m, H))
     sat = 0.6
     du = 0.25 if with_du else None
-    u_prev = 0.3 * rng.standard_normal(m)
+    # the stage-0 box [-sat, sat] & [u_prev - du, u_prev + du] stays at least du / 2 wide: the QP is feasible
+    u_prev = np.clip(0.3 * rng.standard_normal(m), -(sat + 0.125), sat + 0.125)
     return (x_init, X_bm, U_bm, [Q] * H + [Qf], [R] * H, A_ls, B_ls, D_ls, u_prev, sat, du)
 
 
-@pytest.mark.parametrize('c,m', [(4, 1), (4, 2), (8, 2), (9, 2), (16, 3)])
+@pytest.mark.parametrize('c,m', [(4, 1), (4, 2), (8, 2), (9, 2), (16, 3), (16, 1)])
 def test_quad_program_random_instances_all_instantiations(c, m):
     """Every compiled (dim_x, dim_u) kernel against the exact oracle on random QPs: diagonal and full Hermitian costs,
     with and without the rate bound, short and medium horizons.  Tight mode: controls within 1e-8."""

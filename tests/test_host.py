@@ -92,6 +92,15 @@ def test_launch_geometry_without_a_device():
     assert w.value == 14 and c.value == 143     # ceil(2000 / 148) warps per CTA, ceil(2000 / 14) CTAs
     prob.horizon = 400          # does not fit the shared-memory slab: refused, not truncated
     assert lib.m4q_mpc_launch_info(ctypes.byref(prob), 0, ctypes.byref(w), ctypes.byref(c), ctypes.byref(s)) == -1
+    # c = 16: the slab holds the Riccati scratch P [32][34], G [32][42] and K [m][32]
+    gate = _lib.MpcProblem(c=16, m=1, p=1, d=2, horizon=15, n_steps=50, measure_freq=1, lift_mode=_lib.LIFT_PROCESS,
+                           n_targ=66, sat=1.0)      # NOT-gate synthesis on process vectors
+    assert lib.m4q_mpc_launch_info(ctypes.byref(gate), 0, ctypes.byref(w), ctypes.byref(c), ctypes.byref(s)) == 0
+    assert w.value == 8 and c.value == 148      # the MAXW cap of Cfg<16, 1>
+    # CNOT state preparation: order-1 model of three controls, p = 3 monomials
+    cnot = _lib.MpcProblem(c=16, m=3, p=3, d=4, horizon=50, n_steps=200, measure_freq=1, n_targ=251, sat=1.0)
+    assert lib.m4q_mpc_launch_info(ctypes.byref(cnot), 0, ctypes.byref(w), ctypes.byref(c), ctypes.byref(s)) == 0
+    assert w.value == 5 and c.value == 148 and s.value <= 227 * 1024
 
 
 def test_no_cpu_fallback():

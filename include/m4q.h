@@ -219,7 +219,8 @@ int m4q_line_search_batched(int64_t N, int32_t c, int32_t m, int32_t H,
  *   per resident warp (stage records [K | S^-1 | dv | B | D | A_t | x - r] and the state trajectories of the member
  *   the warp is working on; sized for the widest launch on the current device, independent of N).
  *   Environment (measurement aids): M4Q_MAX_WARPS caps the members per CTA; M4Q_L2_PERSIST=0 disables the
- *   persisting-L2 access-policy window that the launch sets on `stream` for the workspaces.
+ *   persisting-L2 access-policy window that the launch sets on `stream` for the workspaces; M4Q_HERM_FACTOR=0 keeps
+ *   every Riccati factorisation in realified coordinates (m4q_mpc_herm_sigma).
  */
 int64_t m4q_mpc_state_bytes(const m4q_mpc_problem *prob_host, int64_t N);
 int64_t m4q_mpc_table_bytes(const m4q_mpc_problem *prob_host);
@@ -230,6 +231,15 @@ int m4q_mpc_closed_loop(const m4q_mpc_problem *prob_host, int64_t N,
                         double *xs, double *us, int32_t *exit_code, int32_t *steps_done,
                         int32_t *qp_count, int32_t *counters, double *fidelity,
                         void *state, void *tables, void *stream);
+
+/* The index involution sigma of the problem's lift (sigma [c]): a Hermitian plant state lifts to x with
+   x[sigma[k]] = conj(x[k]).  Returns 1 if the lift has one, 0 if not, -1 on error.  When the model blocks and costs are
+   sigma-symmetric and a QP's guess trajectory is sigma-conjugate-symmetric, the closed loop runs that QP's Riccati
+   factorisations in the c real coordinates of the Hermitian subspace instead of the 2c realified ones (c = 9). */
+int m4q_mpc_herm_sigma(const m4q_mpc_problem *prob_host, int32_t *sigma);
+/* Byte offset, inside the tables, of two uint64 counters of the last launch: Riccati factorisations run in Hermitian
+   coordinates and in realified coordinates, summed over the members. */
+int64_t m4q_mpc_factor_counts_offset(const m4q_mpc_problem *prob_host);
 
 /* Launch geometry chosen for a problem and N members (N <= 0: the widest launch, which sizes the tables);
    for reporting / roofline accounting. */

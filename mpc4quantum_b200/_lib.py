@@ -56,6 +56,8 @@ SIGNATURES = {
     'm4q_mpc_table_bytes': (c_i64, [ct.POINTER(MpcProblem)]),
     'm4q_mpc_closed_loop': (ct.c_int, [ct.POINTER(MpcProblem), c_i64, c_vp, c_i32, c_vp, c_vp, c_i32, c_i32, c_i32,
                                        c_i32] + [c_vp] * 10),
+    'm4q_mpc_herm_sigma': (ct.c_int, [ct.POINTER(MpcProblem), ct.POINTER(c_i32)]),
+    'm4q_mpc_factor_counts_offset': (c_i64, [ct.POINTER(MpcProblem)]),
     'm4q_mpc_launch_info': (ct.c_int, [ct.POINTER(MpcProblem), c_i64, ct.POINTER(c_i32), ct.POINTER(c_i32),
                                        ct.POINTER(c_i32)]),
     'm4q_hist_fidelity': (ct.c_int, [c_i64, c_vp, c_f64, c_f64, c_i32, c_vp, c_vp]),

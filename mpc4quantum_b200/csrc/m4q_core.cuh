@@ -58,6 +58,40 @@ template <int C_, int M_> struct Cfg {
     static constexpr int KR = (N % 8 == 0) ? N : N + 1;
     static constexpr int LDP = cmin(next_mod(8 * NT, 2, 8), next_mod(8 * NT, 6, 8));
     static constexpr int LDG = cmin(next_mod(8 * GT, 2, 8), next_mod(8 * GT, 6, 8));
+    // the factor runs in Hermitian coordinates (HermCfg) when the QP allows it; the other instantiations keep the
+    // realified factor for every QP
+    static constexpr bool HERM = C_ == 9 && M_ == 2;
+};
+
+// ---------------------------------------------------------------------------------------------------------
+// Factor coordinates of the Hermitian subspace (DESIGN.md section 2.4).  sigma is the index involution of the lift
+// (transpose of vec(rho), ...).  When every model block has N_k[sigma, sigma] = conj(N_k), the costs are sigma-symmetric
+// and the guess trajectory is sigma-conjugate-symmetric, the Riccati recursion leaves the Hermitian subspace
+// {x_sigma(k) = conj(x_k)} (real dimension C) invariant and K_t, S_t^-1, dv_t depend only on P restricted to it.
+// Coordinates (unnormalised, +-1 basis): Re x_k for a fixed point k; (Re x_k + Re x_sk) / 2 and (Im x_k - Im x_sk) / 2
+// for a pair k < sk.  Padded with one zero coordinate to an even count (the P update stores column pairs).
+// ---------------------------------------------------------------------------------------------------------
+template <class CF> struct HermCfg {
+    static constexpr int C = CF::C, N = rup(CF::C, 2), M = CF::M, Q = N + M;
+    static constexpr int NT = cdiv(N, 8), GT = cdiv(Q + 1, 8), TT = cdiv(Q, 8);
+    static constexpr int KR = (N % 8 == 0) ? N : N + 1;
+    static constexpr int LDP = cmin(next_mod(8 * NT, 2, 8), next_mod(8 * NT, 6, 8));
+    static constexpr int LDG = cmin(next_mod(8 * GT, 2, 8), next_mod(8 * GT, 6, 8));
+    // the complex A_t is staged behind the reduced G, inside the realified G buffer
+    static constexpr int ASTAGE = rup(KR * LDG, 2);
+    static_assert(ASTAGE + 2 * C * C <= CF::KR * CF::LDG, "staged A_t does not fit the G buffer");
+    static_assert(KR * LDP <= CF::KR * CF::LDP, "reduced P does not fit the P buffer");
+    static_assert(M * N + N <= M * CF::N, "reduced dv does not fit behind T21");
+};
+// Basis descriptors (ints, built once per launch from sigma, m4q_kernels.cu build_tables):
+//   coordinate a < N:  HB_J1 / HB_J2 [a]: the two realified indices it averages (equal for a fixed point; -1: padding);
+//                      HB_SG [a]: +1 (real part) or -1 (imaginary part: (x_j1 - x_j2) / 2)
+//   realified j < 2C:  HB_CO [j]: the coordinate j belongs to; HB_WT [j]: 2 x its weight in the map back (2, 1, -1, 0);
+//                      HB_PA [j]: the realified index sigma(j) (same part)
+//   HB_OK: 1 when the shared model and the costs are sigma-symmetric (and the reduced factor is enabled)
+template <class CF> struct HermBasis {
+    static constexpr int NR = HermCfg<CF>::N, N = CF::N;
+    static constexpr int J1 = 0, J2 = NR, SG = 2 * NR, CO = 3 * NR, WT = CO + N, PA = WT + N, OK = PA + N, INTS = OK + 1;
 };
 
 // ---------------------------------------------------------------------------------------------------------
@@ -260,6 +294,11 @@ struct QPData {
     double sat;
     int q_diag;           // 1 if every Qbar is diagonal (fast path of the line search / adjoint)
     int Q_soff, Qf_soff, R_soff;   // FUSED: offsets (doubles) of Q, Qf, R in dynamic shared memory
+    // Hermitian coordinates (HermCfg): reduced costs T^T Q T, T^T Qf T (global), basis descriptors (HermBasis) and
+    // whether this QP may use them (herm != 0)
+    const double *Qh, *Qfh;
+    const int *hb;
+    int herm;
 };
 template <bool FUSED> __device__ __forceinline__ QPData localize(const QPData &q) {
     QPData r = q;
@@ -283,6 +322,7 @@ struct Counters {
     int admm, factor, polish, solves;
     int kkt;        // pivoted KKT solves (reported with the polish rounds)
     int sticky;     // kkt_mode 2: a QP of this member broke down numerically in the Riccati path; later QPs skip it
+    int fac_herm, fac_full;   // factorisations in Hermitian / realified coordinates
 };
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -466,27 +506,69 @@ template <class CF> __device__ __forceinline__ double box_hi(const Slab<CF> &s, 
 //   * P_t = Qbar_t + T11 - T21^T K is applied to the accumulator fragments of T11; each lane stores its part of the
 //     upper block triangle and its mirror image, so P stays exactly symmetric.
 // ---------------------------------------------------------------------------------------------------------
-template <class CF, bool FUSED>
+// FC: the factor's coordinates.  FC = CF: the realified state (N = 2C).  FC = HermCfg<CF>: Hermitian coordinates
+// (N = rup(C, 2)); A_t is projected from the complex A_t staged behind G, [B | D] from the ring, the costs are the
+// reduced tables, and K_t, dv_t are mapped back to the realified record layout (halving and sign flips).  One DMMA core
+// for both.
+template <class CF, class FC, bool FUSED>
 __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, const QPData &qp_in, double rho_half,
                                             bool masked, int lane) {
-    constexpr int C = CF::C, N = CF::N, M = CF::M, Q = CF::Q;
-    constexpr int NT = CF::NT, GT = CF::GT, TT = CF::TT, KR = CF::KR, LDP = CF::LDP, LDG = CF::LDG;
+    constexpr int C = CF::C, M = CF::M;
+    constexpr int N = FC::N, Q = FC::Q;
+    constexpr int NT = FC::NT, GT = FC::GT, TT = FC::TT, KR = FC::KR, LDP = FC::LDP, LDG = FC::LDG;
+    constexpr bool RED = FC::N != CF::N;
     constexpr bool LASTNAT = (N % 8 != 0) && (N % 8 <= 4);   // ragged last contraction tile: one k-step of 4 indices
     constexpr int KSTEPS = 2 * NT - (LASTNAT ? 1 : 0);
     using R_ = Rec<CF>;
+    using HB = HermBasis<CF>;
     const Slab<CF> s = slab_view<CF>(sr);
     const StageOps ops = localize<FUSED>(ops_in);
     const QPData qp = localize<FUSED>(qp_in);
     const int H = sr.H;
     const int g8 = lane >> 2, c4 = lane & 3;   // fragment coordinates of this lane
+    const double *Qfac = RED ? qp.Qh : qp.Q, *Qffac = RED ? qp.Qfh : qp.Qf;
     // P <- Qf with zero padding; G zeroed once (padding rows / columns are never written afterwards)
 #pragma unroll 1
     for (int e = lane; e < KR * LDP; e += 32) {
         const int i = e / LDP, j = e % LDP;
-        s.P[e] = (i < N && j < N) ? qp.Qf[i * N + j] : 0.0;
+        s.P[e] = (i < N && j < N) ? Qffac[i * N + j] : 0.0;
     }
 #pragma unroll 1
     for (int e = lane; e < KR * LDG; e += 32) s.AB[e] = 0.0;
+    // Hermitian coordinates: what this lane projects and maps back (constant over the stages)
+    constexpr int NEA = RED ? cdiv(C * C, 32) : 1;
+    int a_o1[NEA], a_o2[NEA], a_g[NEA];
+    double a_s2[NEA], a_sg[NEA];
+    bool a_re[NEA];
+    int h_j1 = 0, h_j2 = 0, h_co = 0;
+    double h_sg = 0.0, h_wt = 0.0;
+    double2 *astage = reinterpret_cast<double2 *>(s.AB + HermCfg<CF>::ASTAGE);
+    if constexpr (RED) {
+#pragma unroll
+        for (int q = 0; q < NEA; ++q) {
+            // entry (a, b) of A~ = T^+ A_t T: column b of A_t T is A[:, kc] + s2 A[:, kc2] (times i for an imaginary
+            // coordinate), read at the representative row kr of coordinate a (real or imaginary part)
+            const int e = lane + 32 * q, a = e < C * C ? e / C : 0, b = e < C * C ? e % C : 0;
+            const int r1 = qp.hb[HB::J1 + a], c1 = qp.hb[HB::J1 + b], c2 = qp.hb[HB::J2 + b];
+            const bool row_im = r1 >= C, col_im = c1 >= C;
+            const int kr = r1 % C, kc = c1 % C, kc2 = c2 % C;
+            a_o1[q] = kr * C + kc;
+            a_o2[q] = kr * C + kc2;
+            a_s2[q] = c1 == c2 ? 0.0 : (double)qp.hb[HB::SG + b];
+            a_re[q] = row_im == col_im;
+            a_sg[q] = (col_im && !row_im) ? -1.0 : 1.0;
+            a_g[q] = e < C * C ? a * LDG + b : -1;
+        }
+        if (lane < C) {
+            h_j1 = qp.hb[HB::J1 + lane];
+            h_j2 = qp.hb[HB::J2 + lane];
+            h_sg = (double)qp.hb[HB::SG + lane];
+        }
+        if (lane < CF::N) {
+            h_co = qp.hb[HB::CO + lane];
+            h_wt = 0.5 * (double)qp.hb[HB::WT + lane];
+        }
+    }
     // where the entries of A_t this lane forms go: element e = lane + 32 q of the row-major C x C block
     constexpr int NE = cdiv(C * C, 32);
     int g_off[NE], r_off[NE];
@@ -529,20 +611,43 @@ __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, 
 #pragma unroll
             for (int q = 0; q < NE; ++q) {
                 if (g_off[q] >= 0) {
-                    double *g = s.AB + g_off[q];
-                    g[0] = ar[q];
-                    g[C] = -ai[q];
-                    g[C * LDG] = ai[q];
-                    g[C * LDG + C] = ar[q];
+                    if constexpr (RED) {
+                        astage[lane + 32 * q] = make_double2(ar[q], ai[q]);
+                    } else {
+                        double *g = s.AB + g_off[q];
+                        g[0] = ar[q];
+                        g[C] = -ai[q];
+                        g[C * LDG] = ai[q];
+                        g[C * LDG + C] = ar[q];
+                    }
                     reinterpret_cast<double2 *>(rec + R_::AT)[r_off[q]] = make_double2(ar[q], ai[q]);
                 }
+            }
+        }
+        if constexpr (RED) {
+            __syncwarp();   // the complex A_t is staged
+#pragma unroll
+            for (int q = 0; q < NEA; ++q) {
+                const double2 z1 = astage[a_o1[q]], z2 = astage[a_o2[q]];
+                const double zr = fma(a_s2[q], z2.x, z1.x), zi = fma(a_s2[q], z2.y, z1.y);
+                if (a_g[q] >= 0) s.AB[a_g[q]] = a_re[q] ? zr : a_sg[q] * zi;
             }
         }
         // B~ into G[:, N:Q], D~ into G[:, Q]: lane k < N owns row k; the working set of the stage is read once
         int mk[M];
 #pragma unroll
         for (int i = 0; i < M; ++i) mk[i] = masked ? s.mask[t * M + i] : 0;
-        if (lane < N) {
+        if (RED && lane < C) {
+            // coordinate lane of B_t, D_t: (x_j1 +- x_j2) / 2 (a fixed point: j1 == j2, +)
+            double dt = 0.5 * fma(h_sg, Dt[h_j2], Dt[h_j1]);
+#pragma unroll
+            for (int i = 0; i < M; ++i) {
+                const double b = 0.5 * fma(h_sg, Bt[R_::pair(i, h_j2)], Bt[R_::pair(i, h_j1)]);
+                s.AB[lane * LDG + N + i] = mk[i] ? 0.0 : b;
+                if (mk[i]) dt = fma(b, mk[i] == 1 ? box_lo(s, qp.sat, t, i) : box_hi(s, qp.sat, t, i), dt);
+            }
+            s.AB[lane * LDG + Q] = dt;
+        } else if (!RED && lane < N) {
             double dt = Dt[lane];
 #pragma unroll
             for (int i = 0; i < M; ++i) {
@@ -596,11 +701,13 @@ __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, 
             }
         }
         // dv_t = P_{t+1} D~_t = row Q of W^T: held by the lanes with g8 == Q % 8, columns mi*8 + 2 c4 + {0, 1}
+        // (Hermitian coordinates: to the scratch behind T21, mapped back below)
+        double *dvb = s.T21 + M * N;
         if (g8 == Q % 8) {
 #pragma unroll
             for (int mi = 0; mi < NT; ++mi) {
                 const int j = mi * 8 + 2 * c4;
-                if (j < N) *reinterpret_cast<double2 *>(rec + R_::DV + j) = make_double2(w[Q / 8][mi][0], w[Q / 8][mi][1]);
+                if (j < N) *reinterpret_cast<double2 *>((RED ? dvb : rec + R_::DV) + j) = make_double2(w[Q / 8][mi][0], w[Q / 8][mi][1]);
             }
         }
         // ---- T = W^T G, upper block triangle of the leading Q x Q part: A operand = the accumulators of W^T
@@ -686,13 +793,19 @@ __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, 
                 double kv = 0.0;
 #pragma unroll
                 for (int b = 0; b < M; ++b) kv = fma(Si[a][b], s.T21[b * N + lane], kv);
-                rec[R_::K + R_::pair(a, lane)] = kv;
+                if (!RED) rec[R_::K + R_::pair(a, lane)] = kv;
                 s.W[a * N + lane] = kv;
             }
         }
         __syncwarp();
+        if (RED && lane < CF::N) {
+            // back to the realified record: x_j = w_j y_co(j) with w_j in {1, 1/2, -1/2, 0}
+#pragma unroll
+            for (int a = 0; a < M; ++a) rec[R_::K + R_::pair(a, lane)] = h_wt == 0.0 ? 0.0 : h_wt * s.W[a * N + h_co];
+            rec[R_::DV + lane] = h_wt == 0.0 ? 0.0 : h_wt * dvb[h_co];
+        }
         // ---- P_t = Qbar_t + T11 - T21^T K on the accumulator fragments; upper block triangle + mirror image
-        const double *Qt = qp.Q + t * qp.q_stride;
+        const double *Qt = Qfac + t * qp.q_stride;
 #pragma unroll
         for (int qi = 0; qi < NT; ++qi) {
             const int i = qi * 8 + g8;
@@ -744,6 +857,22 @@ __device__ __noinline__ void riccati_factor(SlabRef sr, const StageOps &ops_in, 
         }
     }
     __syncwarp();
+}
+
+// The factor a QP runs: Hermitian coordinates when the instantiation has them and the QP's premise holds (qp.herm, set
+// per QP by the closed loop), else realified.  Counted per member.
+template <class CF, bool FUSED>
+__device__ __forceinline__ void factor(SlabRef sr, const StageOps &ops, const QPData &qp, double rho_half, bool masked,
+                                       int lane, Counters &cnt) {
+    if constexpr (CF::HERM && FUSED) {
+        if (qp.herm) {
+            riccati_factor<CF, HermCfg<CF>, FUSED>(sr, ops, qp, rho_half, masked, lane);
+            cnt.fac_herm++;
+            return;
+        }
+    }
+    riccati_factor<CF, CF, FUSED>(sr, ops, qp, rho_half, masked, lane);
+    cnt.fac_full++;
 }
 
 // stage record t of the workspace -> slot (t & 1) of the record ring in the [P | G] buffers
@@ -1048,7 +1177,7 @@ __device__ __noinline__ void admm_block(SlabRef sr, const StageOps &ops_in, cons
             // is rescaled by sqrt(normalised primal residual / normalised dual residual) when that ratio is far from
             // one, the scaled dual y follows, and the Riccati factorisation is redone with the new rho.
             double rho = set.rho, rh = rho_half;
-            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
+            factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane, cnt);
             cnt.factor++;
             int next_check = 5;
             for (int it = 0; it < set.max_admm; ++it) {
@@ -1091,7 +1220,7 @@ __device__ __noinline__ void admm_block(SlabRef sr, const StageOps &ops_in, cons
                         __syncwarp();
                         rho = rho_new;
                         rh = 0.5 * rho;
-                        riccati_factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane);
+                        factor<CF, FUSED>(sr, ops_in, qp_in, rh, false, lane, cnt);
                         cnt.factor++;
                     }
                 }
@@ -1150,7 +1279,8 @@ __device__ int qp_solve(SlabRef sr, const StageOps &ops_in, const QPData &qp_in,
         if (kkt_ok && ((set.kkt_mode >= 2 && cnt.sticky) || set.kkt_mode >= 4)) {
             // an earlier QP of this member needed the pivoted KKT solve (cost-to-go beyond fp64: order-1 model at long
             // horizons): go straight to it.  One factor call forms the stage operators A_t in the records.
-            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, 0.0, false, lane);
+            riccati_factor<CF, CF, FUSED>(sr, ops_in, qp_in, 0.0, false, lane);
+            cnt.fac_full++;
             status = kkt_active_set<CF, FUSED>(sr, qp_in, set, lane, cnt);
             break;
         }
@@ -1197,7 +1327,7 @@ __device__ int qp_solve(SlabRef sr, const StageOps &ops_in, const QPData &qp_in,
         bool certified = false;
         bool numeric = false;   // the rounds ended on a settled working set whose solve is not stationary, or not finite
         for (int round = 0; round < set.max_polish; ++round) {
-            riccati_factor<CF, FUSED>(sr, ops_in, qp_in, 0.0, true, lane);
+            factor<CF, FUSED>(sr, ops_in, qp_in, 0.0, true, lane, cnt);
             cnt.factor++;
             cnt.polish++;
             x_nonfinite = riccati_solve<CF, FUSED>(sr, qp_in, 0.0, SWEEP_POLISH, true, lane) != 0.0;
@@ -1381,8 +1511,10 @@ __device__ double qp_objective(const SlabRef &sr, const QPData &qp, int lane) {
 // x_t comes from the workspace one stage ahead (register prefetch); the vector and the derivative weights are
 // double-buffered, so one warp sync per stage.
 // ---------------------------------------------------------------------------------------------------------
+// hb != nullptr: also checks that Xg is sigma-conjugate-symmetric (x_sigma(k) = conj(x_k), HermBasis) over all H + 1
+// stages to 1e-12 of its largest entry -- the premise of the factor in Hermitian coordinates; returns 1 if it is.
 template <class CF, bool FUSED>
-__device__ __noinline__ void linearize(SlabRef sr, const StageOps &model_in, const int *pow, int lane) {
+__device__ __noinline__ int linearize(SlabRef sr, const StageOps &model_in, const int *pow, int lane, const int *hb) {
     constexpr int C = CF::C, N = CF::N, M = CF::M;
     using R_ = Rec<CF>;
     const Slab<CF> s = slab_view<CF>(sr);
@@ -1395,6 +1527,18 @@ __device__ __noinline__ void linearize(SlabRef sr, const StageOps &model_in, con
     const int r = im ? lane - C : lane;
     const double sgn = im ? 1.0 : -1.0;
     double x_n = act ? Xg[lane] : 0.0;
+    // sigma check: the partner lane holds x_sigma(j), equal to x_j (real part) or -x_j (imaginary part)
+    const bool chk = hb != nullptr;
+    const int pa = (chk && act) ? hb[HermBasis<CF>::PA + lane] : lane;
+    const double hs = im ? -1.0 : 1.0;
+    double hdev = 0.0, hmax = 0.0;
+    bool hnf = false;
+    auto herm_stage = [&](double x) {
+        const double xp = __shfl_sync(FULL, x, pa);
+        hdev = fmax(hdev, fabs(xp - hs * x));
+        hmax = fmax(hmax, fabs(x));
+        hnf |= !isfinite(x);
+    };
     // order-1 library (phi_k = u_k): the derivative weights are the identity and need not be tabulated per stage
     bool first_order = p == M;
     if (first_order) {
@@ -1405,6 +1549,7 @@ __device__ __noinline__ void linearize(SlabRef sr, const StageOps &model_in, con
     for (int t = 0; t < H; ++t) {
         double *dco = s.scr + (t & 1) * (p * M);   // [p][M]
         double *vec = (t & 1) ? s.vb : s.va;
+        if (chk) herm_stage(x_n);
         if (act) {
             vec[lane] = x_n;
             if (t + 1 < H) x_n = Xg[(t + 1) * N + lane];
@@ -1476,6 +1621,10 @@ __device__ __noinline__ void linearize(SlabRef sr, const StageOps &model_in, con
         }
     }
     __syncwarp();
+    if (!chk) return 0;
+    herm_stage(act ? Xg[H * N + lane] : 0.0);
+    const double tol = 1e-12 * warp_max(hmax);
+    return !__any_sync(FULL, hnf || !(hdev <= tol));
 }
 
 // ---------------------------------------------------------------------------------------------------------

@@ -32,7 +32,7 @@ static int fail(const std::string &msg) {
 // Layout in doubles; offsets from TableLayout.
 // ---------------------------------------------------------------------------------------------------------
 struct TableLayout {
-    int Qr, Qfr, Rr, r, qlin, qlinf, ub, Rub, flags, total;
+    int Qr, Qfr, Rr, r, qlin, qlinf, ub, Rub, flags, hq, hqf, hb, total;
     __host__ __device__ TableLayout(int N, int M, int n_targ) {
         int o = 0;
         auto take = [&](int cnt) {
@@ -48,7 +48,13 @@ struct TableLayout {
         qlinf = take(n_targ * N);
         ub = take(n_targ * M);
         Rub = take(n_targ * M);
-        flags = take(4);   // [0] q_diag, [1..2] work counter (as int)
+        flags = take(4);   // [0] q_diag, [1] work counter (as int), [2..3] factorisations in Hermitian / realified
+                           // coordinates (unsigned 64-bit, summed over the members of the launch)
+        // Hermitian coordinates (HermCfg, HermBasis in m4q_core.cuh): reduced costs T^T Q T, T^T Qf T, basis descriptors
+        const int NR = rup(N / 2, 2);
+        hq = take(NR * NR);
+        hqf = take(NR * NR);
+        hb = take(cdiv(3 * NR + 3 * N + 1, 2));
         total = o;
     }
 };
@@ -64,8 +70,28 @@ __device__ __forceinline__ double realified_sym(const double2 *Qc, int C, int i,
     return 0.5 * (entry(i, j) + entry(j, i));
 }
 
+// sigma of the lift (m4q_mpc_herm_sigma); ok = 0: the factor stays realified
+struct HermSigma {
+    int ok;
+    int sig[32];
+};
+
+// Largest deviation of a model block from sigma-conjugate symmetry, N[s(i)][s(j)] = conj(N[i][j]), against the tolerance:
+// true if symmetric.  The device Taylor discretisation sums the products of an entry and of its partner in different
+// orders (q and s(q)), so the blocks it produces are symmetric to a few ulp, not bit for bit: the tolerance is 16 ulp of
+// the block's largest entry.  The same comparisons run for shared (build_tables) and per-member models (mpc_kernel),
+// so a member gets the same factor whichever way its model arrives.
+__device__ __forceinline__ double herm_block_scale(double2 v) { return fmax(fabs(v.x), fabs(v.y)); }
+__device__ __forceinline__ bool herm_entry_ok(const double2 *blk, const int *sig, int C, int e, double scale) {
+    const int i = e / C, j = e % C;
+    const double2 a = blk[e], b = blk[sig[i] * C + sig[j]];
+    const double tol = 16.0 * 2.220446049250313e-16 * scale;
+    return fabs(b.x - a.x) <= tol && fabs(b.y + a.y) <= tol;
+}
+
 __global__ void build_tables(int C, int M, int n_targ, const double2 *Q, const double2 *Qf, const double *R,
-                             const double2 *X_targ, const double *U_targ, double *tab) {
+                             const double2 *X_targ, const double *U_targ, double *tab, HermSigma hs,
+                             const double2 *A_blocks, int nblk) {
     const int N = 2 * C;
     const TableLayout L(N, M, n_targ);
     const int tid = threadIdx.x, nt = blockDim.x;
@@ -114,6 +140,85 @@ __global__ void build_tables(int C, int M, int n_targ, const double2 *Q, const d
         int *ctr = reinterpret_cast<int *>(tab + L.flags + 1);
         ctr[0] = 0;
         ctr[1] = 0;
+        unsigned long long *fc = reinterpret_cast<unsigned long long *>(tab + L.flags + 2);
+        fc[0] = 0;
+        fc[1] = 0;
+        // basis of the Hermitian coordinates (HermBasis): a fixed point k of sigma gives Re x_k; a pair k < s(k) gives
+        // (Re x_k + Re x_sk) / 2 and (Im x_k - Im x_sk) / 2
+        const int NR = rup(C, 2);
+        int *hb = reinterpret_cast<int *>(tab + L.hb);
+        int *J1 = hb, *J2 = hb + NR, *SG = hb + 2 * NR, *CO = hb + 3 * NR, *WT = CO + N, *PA = WT + N, *OK = PA + N;
+        for (int a = 0; a < NR; ++a) J1[a] = J2[a] = SG[a] = 0;
+        int a = 0;
+        bool ok = hs.ok != 0;
+        for (int k = 0; k < C && ok; ++k) {
+            const int sk = hs.sig[k];
+            ok &= sk >= 0 && sk < C && hs.sig[sk] == k;
+            if (!ok) break;
+            PA[k] = sk;
+            PA[C + k] = C + sk;
+            if (sk == k) {
+                J1[a] = J2[a] = k;
+                SG[a] = 1;
+                CO[k] = CO[C + k] = a;
+                WT[k] = 2;
+                WT[C + k] = 0;
+                ++a;
+            } else if (k < sk) {
+                J1[a] = k;
+                J2[a] = sk;
+                SG[a] = 1;
+                CO[k] = CO[sk] = a;
+                WT[k] = WT[sk] = 1;
+                ++a;
+                J1[a] = C + k;
+                J2[a] = C + sk;
+                SG[a] = -1;
+                CO[C + k] = CO[C + sk] = a;
+                WT[C + k] = 1;
+                WT[C + sk] = -1;
+                ++a;
+            }
+        }
+        if (!ok)
+            for (int j = 0; j < N; ++j) {
+                CO[j] = WT[j] = 0;
+                PA[j] = j;
+            }
+        // the premise shared by every QP of the launch: sigma-symmetric costs (exact) and shared model blocks
+        for (int i = 0; i < N && ok; ++i)
+            for (int j = 0; j < N; ++j) {
+                const int pi = PA[i], pj = PA[j];
+                const double sg = ((i < C) == (j < C)) ? 1.0 : -1.0;
+                ok &= tab[L.Qr + pi * N + pj] * sg == tab[L.Qr + i * N + j] && tab[L.Qfr + pi * N + pj] * sg == tab[L.Qfr + i * N + j];
+            }
+        for (int kb = 0; kb < nblk && ok && A_blocks; ++kb) {
+            const double2 *blk = A_blocks + (size_t)kb * C * C;
+            double scale = 0.0;
+            for (int e = 0; e < C * C; ++e) scale = fmax(scale, herm_block_scale(blk[e]));
+            for (int e = 0; e < C * C; ++e) ok &= herm_entry_ok(blk, hs.sig, C, e, scale);
+        }
+        *OK = ok ? 1 : 0;
+    }
+    __syncthreads();
+    // reduced costs T^T Q T: coordinate a is x_J1 + SG x_J2 (x_J1 alone for a fixed point); padding rows stay zero
+    const int NR = rup(C, 2);
+    const int *hb = reinterpret_cast<const int *>(tab + L.hb);
+    for (int e = tid; e < NR * NR; e += nt) {
+        const int a = e / NR, b = e % NR;
+        double q = 0.0, qf = 0.0;
+        if (a < C && b < C) {
+            const int ja[2] = {hb[a], hb[NR + a]}, jb[2] = {hb[b], hb[NR + b]};
+            const double wa[2] = {1.0, ja[0] == ja[1] ? 0.0 : (double)hb[2 * NR + a]};
+            const double wb[2] = {1.0, jb[0] == jb[1] ? 0.0 : (double)hb[2 * NR + b]};
+            for (int u = 0; u < 2; ++u)
+                for (int v = 0; v < 2; ++v) {
+                    q = fma(wa[u] * wb[v], tab[L.Qr + ja[u] * N + jb[v]], q);
+                    qf = fma(wa[u] * wb[v], tab[L.Qfr + ja[u] * N + jb[v]], qf);
+                }
+        }
+        tab[L.hq + e] = q;
+        tab[L.hqf + e] = qf;
     }
 }
 
@@ -453,6 +558,9 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
 
     int *work = reinterpret_cast<int *>(a.tab + L.flags + 1);
     const int q_diag = a.tab[L.flags] != 0.0;
+    // factor in Hermitian coordinates: instantiation, launch-wide premise (build_tables), then per member and per QP
+    const int *hb = reinterpret_cast<const int *>(a.tab + L.hb);
+    const bool herm_launch = CF::HERM && !EXACT && hb[HermBasis<CF>::OK] != 0;
     const int persist = Slab<CF>::persistent_doubles(H, cmax(dd, C));
 
     for (;;) {
@@ -461,7 +569,8 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
         k = __shfl_sync(FULL, k, 0);
         if (k >= a.n_members) break;
 
-        Counters cnt = {0, 0, 0, 0};
+        Counters cnt = {};
+        bool herm_member = herm_launch;
         int exit_code = 0;
         double2 *xs_k = a.xs + (size_t)k * xdim * (S + 1);
         double *us_k = a.us + (size_t)k * M * S;
@@ -473,6 +582,22 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
 #pragma unroll 1
             for (int e = lane; e < a.nblk * C * C; e += 32) mine[e] = src[e];
             __syncwarp();
+            if (herm_member) {
+                // the member's own blocks must be sigma-symmetric too (same test as build_tables)
+                const int *sig = hb + HermBasis<CF>::PA;   // sigma on the real parts
+                bool ok = true;
+#pragma unroll 1
+                for (int kb = 0; kb < a.nblk; ++kb) {
+                    const double2 *blk = mine + kb * C * C;
+                    double scale = 0.0;
+#pragma unroll 1
+                    for (int e = lane; e < C * C; e += 32) scale = fmax(scale, herm_block_scale(blk[e]));
+                    scale = warp_max(scale);
+#pragma unroll 1
+                    for (int e = lane; e < C * C; e += 32) ok &= herm_entry_ok(blk, sig, C, e, scale);
+                }
+                herm_member = __all_sync(FULL, ok);
+            }
         }
 
         // ---- initial or restored loop state
@@ -537,6 +662,10 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
                 qp.Q_soff = 2 * a.nblk * C * C;
                 qp.Qf_soff = qp.Q_soff + N * N;
                 qp.R_soff = qp.Qf_soff + N * N;
+                qp.Qh = a.tab + L.hq;
+                qp.Qfh = a.tab + L.hqf;
+                qp.hb = hb;
+                qp.herm = 0;
 
                 // measured state -> model space: the QP's initial condition (mpc.py:187)
                 lift_state<CF>(a.external_plant ? M4Q_LIFT_IDENTITY : a.lift_mode, d, xcur, s.x0, lane);
@@ -578,7 +707,8 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
                         dense.first_order = 0;
                         status = qp_solve<CF, false>(sr, dense, qp, a.set, lane, cnt);
                     } else {
-                        linearize<CF, true>(sr, model, pow, lane);                  // mpc.py:175
+                        // mpc.py:175; the premise of the Hermitian factor is checked on this QP's guess trajectory
+                        qp.herm = linearize<CF, true>(sr, model, pow, lane, herm_member ? hb : nullptr);
                         status = qp_solve<CF, true>(sr, model, qp, a.set, lane, cnt);   // mpc.py:189
                     }
                     if (status != 0) {
@@ -744,6 +874,9 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
                 c[2] += cnt.polish + cnt.kkt;
                 c[3] += cnt.solves;
             }
+            unsigned long long *fc = reinterpret_cast<unsigned long long *>(a.tab + L.flags + 2);
+            if (cnt.fac_herm) atomicAdd(fc, (unsigned long long)cnt.fac_herm);
+            if (cnt.fac_full) atomicAdd(fc + 1, (unsigned long long)cnt.fac_full);
         }
         if (a.fidelity && !a.external_plant && a.fid_vec) {
             const double f = fidelity_of<CF>(a.lift_mode, d, a.fid_vec, xcur, s.va, lane);
@@ -1710,6 +1843,46 @@ template <class CF> static int mpc_geometry(const m4q_mpc_problem *p, long long 
     return plan(mpc_kernel<CF, false>, CF::MAXW, slab, mpc_shared_doubles<CF>(p->p + 1), n, have_device, g);
 }
 
+// The index involution sigma of the lift: the model state of a Hermitian plant state satisfies x_sigma(k) = conj(x_k).
+//   identity lift, vec(rho) of a dA x dA matrix (external plant: c must be a square): transpose
+//   trunc32: the 2 x 2 block, transpose;  coupled: transpose inside each stacked dA x dA block
+//   process, vec(U (x) U^*): swap of the two tensor factors, (i d + k) d^2 + (j d + l) <-> (k d + i) d^2 + (l d + j)
+// Returns false when there is none to use (exact model mode: the factor stays realified).
+static bool herm_sigma(const m4q_mpc_problem *p, int *sig) {
+    const int c = p->c, d = p->d;
+    if (p->model_mode != M4Q_MODEL_TAYLOR || c < 1 || c > 32) return false;
+    auto transpose = [&](int off, int n) {
+        for (int i = 0; i < n; ++i)
+            for (int j = 0; j < n; ++j) sig[off + i * n + j] = off + j * n + i;
+    };
+    if (p->lift_mode == M4Q_LIFT_IDENTITY) {
+        int n = 0;
+        while ((n + 1) * (n + 1) <= c) ++n;
+        if (n * n != c) return false;
+        transpose(0, n);
+    } else if (p->lift_mode == M4Q_LIFT_TRUNC32) {
+        if (c != 4) return false;
+        transpose(0, 2);
+    } else if (p->lift_mode == M4Q_LIFT_COUPLED) {
+        int n = 0;
+        while (2 * (n + 1) * (n + 1) <= c) ++n;
+        if (2 * n * n != c) return false;
+        transpose(0, n);
+        transpose(n * n, n);
+    } else if (p->lift_mode == M4Q_LIFT_PROCESS) {
+        if (d < 1 || d * d * d * d != c) return false;
+        const int d2 = d * d;
+        for (int row = 0; row < d2; ++row)
+            for (int col = 0; col < d2; ++col) {
+                const int i = row / d, k = row % d, j = col / d, l = col % d;
+                sig[row * d2 + col] = (k * d + i) * d2 + (l * d + j);
+            }
+    } else {
+        return false;
+    }
+    return true;
+}
+
 template <class CF>
 static int launch_mpc(const m4q_mpc_problem *p, long long n, const MpcArgs &base, cudaStream_t st) {
     Geometry g;
@@ -1719,9 +1892,16 @@ static int launch_mpc(const m4q_mpc_problem *p, long long n, const MpcArgs &base
     a.shared_doubles = g.shared_doubles;
     // per-warp workspaces follow the shared tables (sized by m4q_mpc_table_bytes for the widest launch)
     a.ws = a.tab + rup(TableLayout(CF::N, CF::M, p->n_targ).total, 2);
+    // M4Q_HERM_FACTOR=0 keeps every factorisation realified (measurement aid, read per launch)
+    HermSigma hs;
+    memset(&hs, 0, sizeof(hs));
+    const char *hv = getenv("M4Q_HERM_FACTOR");
+    hs.ok = CF::HERM && (!hv || atoi(hv) != 0) && herm_sigma(p, hs.sig);
     build_tables<<<1, 256, 0, st>>>(CF::C, CF::M, p->n_targ, reinterpret_cast<const double2 *>(p->Q),
                                     reinterpret_cast<const double2 *>(p->Qf), p->R,
-                                    reinterpret_cast<const double2 *>(p->X_targ), p->U_targ, a.tab);
+                                    reinterpret_cast<const double2 *>(p->X_targ), p->U_targ, a.tab, hs,
+                                    p->model_per_member ? nullptr : reinterpret_cast<const double2 *>(p->A_blocks),
+                                    p->p + 1);
     M4Q_CUDA(cudaGetLastError());
     // The workspaces are rewritten every QP; ask L2 to keep them (persisting lines) instead of writing them back to
     // HBM.  Best effort: M4Q_L2_PERSIST=0 switches it off, failures are ignored.
@@ -2073,6 +2253,20 @@ int64_t m4q_mpc_table_bytes(const m4q_mpc_problem *p) {
         if (p->qp.kkt_fallback > 0 && p->qp.polish) ws += (long long)g.ctas * g.warps * Kkt<CF>::doubles(p->horizon);
     });
     return (int64_t)sizeof(double) * (rup(TableLayout(2 * p->c, p->m, p->n_targ).total, 2) + ws);
+}
+
+int m4q_mpc_herm_sigma(const m4q_mpc_problem *p, int32_t *sigma) {
+    if (check_problem(p) != 0) return -1;
+    int sig[32];
+    if (!herm_sigma(p, sig)) return 0;
+    if (sigma)
+        for (int k = 0; k < p->c; ++k) sigma[k] = sig[k];
+    return 1;
+}
+
+int64_t m4q_mpc_factor_counts_offset(const m4q_mpc_problem *p) {
+    if (check_problem(p) != 0) return -1;
+    return (int64_t)sizeof(double) * (TableLayout(2 * p->c, p->m, p->n_targ).flags + 2);
 }
 
 int m4q_mpc_launch_info(const m4q_mpc_problem *p, int64_t N, int32_t *warps_per_cta, int32_t *ctas, int32_t *smem_bytes) {

@@ -270,6 +270,23 @@ class ClosedLoopPlan:
         _lib.check(_lib.lib().m4q_mpc_launch_info(ct.byref(self.prob), int(n), ct.byref(w), ct.byref(c), ct.byref(s)))
         return dict(warps_per_cta=w.value, ctas=c.value, smem_bytes=s.value)
 
+    def herm_sigma(self):
+        """The lift's index involution sigma (list of c ints), or None when the lift has none."""
+        sig = (_lib.c_i32 * max(int(self.prob.c), 1))()
+        r = _lib.lib().m4q_mpc_herm_sigma(ct.byref(self.prob), sig)
+        if r < 0:
+            _lib.check(-1)
+        return list(sig[:int(self.prob.c)]) if r == 1 else None
+
+    def factor_counts(self):
+        """Riccati factorisations of the last launch: dict(herm=..., full=...), Hermitian and realified coordinates.
+        Synchronises the current stream."""
+        off = int(_lib.lib().m4q_mpc_factor_counts_offset(ct.byref(self.prob)))
+        if off < 0:
+            _lib.check(-1)
+        v = self.tables[off:off + 16].cpu().numpy().view(np.uint64)
+        return dict(herm=int(v[0]), full=int(v[1]))
+
     def run(self, x0, H0=None, H1=None, n=None, x0_shared=False, shared_hamiltonian=False, step_begin=0,
             step_end=None, stream=None, noise_sigma=0.0, noise_seed=0, member_offset=0, streaming=None,
             fidelity_sqrt=False):

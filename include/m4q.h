@@ -119,7 +119,7 @@ typedef struct {
 int m4q_version(void);
 const char *m4q_last_error(void);
 
-/* 1 if the (c, m) pair has a compiled kernel instantiation. */
+/* 1 if the (c, m) pair has a compiled kernel instantiation: c in {4, 8, 9, 16} with m in {1, 2, 3, 4}. */
 int m4q_supported(int32_t c, int32_t m);
 
 /*

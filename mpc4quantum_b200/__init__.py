@@ -9,5 +9,6 @@ from .model import *        # noqa: F401,F403
 from .mpc import *          # noqa: F401,F403
 from .vectorize import *    # noqa: F401,F403
 from . import experiment, linearize, model, optimize, vectorize  # noqa: F401  (`mpc` names the function, as upstream)
+from ._lib import supported_shapes  # noqa: F401
 
 __version__ = '0.1.0'

@@ -84,6 +84,26 @@ def lib():
     return _lib
 
 
+_shapes = None
+
+
+def supported_shapes():
+    """The (dim_x, dim_u) pairs the library has kernels for, as m4q_supported reports them (every dim_x <= 32 and
+    dim_u <= 32 is asked once)."""
+    global _shapes
+    if _shapes is None:
+        handle = lib()
+        _shapes = [(c, m) for c in range(1, 33) for m in range(1, 33) if handle.m4q_supported(c, m)]
+    return list(_shapes)
+
+
+def require_shape(c, m):
+    """Raise NotImplementedError, naming the compiled pairs, unless (c, m) = (dim_x, dim_u) has kernels."""
+    if not lib().m4q_supported(c, m):
+        raise NotImplementedError('no compiled kernel for (dim_x, dim_u) = (%d, %d); the compiled pairs are %s'
+                                  % (c, m, ', '.join('(%d, %d)' % s for s in supported_shapes())))
+
+
 def check(rc):
     if rc != 0:
         raise RuntimeError('libm4q: ' + lib().m4q_last_error().decode())

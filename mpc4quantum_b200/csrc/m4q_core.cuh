@@ -40,14 +40,14 @@ __host__ __device__ constexpr int cmin(int a, int b) { return a < b ? a : b; }
 #ifndef M4Q_MAXW_4
 #define M4Q_MAXW_4 32
 #endif
-template <int C_, int M_> struct Tiles { static constexpr int MAXW = C_ == 4 ? M4Q_MAXW_4 : 16; };   // C = 4: 32 warps x 64 registers (+18 % on the qubit, spills and all); else 16 x 128
+// C = 4: 32 warps x 64 registers (+18 % on the qubit, spills and all); C = 16: 8 x 255 (the factor and sweeps of
+// N = 32 do not fit 128 registers); else 16 x 128
+template <int C_, int M_> struct Tiles { static constexpr int MAXW = C_ == 4 ? M4Q_MAXW_4 : C_ == 16 ? 8 : 16; };
 #ifndef M4Q_MAXW_92
 #define M4Q_MAXW_92 16
 #endif
 template <> struct Tiles<9, 2> { static constexpr int MAXW = M4Q_MAXW_92; };   // 12: 3 warps per scheduler, 168 registers, no spills
 template <> struct Tiles<8, 2> { static constexpr int MAXW = 16; };   // 15 fit; measured faster than 12 x 168 registers
-template <> struct Tiles<16, 3> { static constexpr int MAXW = 8; };
-template <> struct Tiles<16, 1> { static constexpr int MAXW = 8; };
 
 template <int C_, int M_> struct Cfg {
     static constexpr int C = C_, N = 2 * C_, M = M_, Q = N + M_;
@@ -77,11 +77,12 @@ template <class CF> struct HermCfg {
     static constexpr int KR = (N % 8 == 0) ? N : N + 1;
     static constexpr int LDP = cmin(next_mod(8 * NT, 2, 8), next_mod(8 * NT, 6, 8));
     static constexpr int LDG = cmin(next_mod(8 * GT, 2, 8), next_mod(8 * GT, 6, 8));
-    // the complex A_t is staged behind the reduced G, inside the realified G buffer
+    // the complex A_t is staged behind the reduced G, inside the realified G buffer.  Only instantiations with
+    // CF::HERM run this factor; riccati_factor instantiates HermCfg for every CF, so the layout checks bind only there.
     static constexpr int ASTAGE = rup(KR * LDG, 2);
-    static_assert(ASTAGE + 2 * C * C <= CF::KR * CF::LDG, "staged A_t does not fit the G buffer");
-    static_assert(KR * LDP <= CF::KR * CF::LDP, "reduced P does not fit the P buffer");
-    static_assert(M * N + N <= M * CF::N, "reduced dv does not fit behind T21");
+    static_assert(!CF::HERM || ASTAGE + 2 * C * C <= CF::KR * CF::LDG, "staged A_t does not fit the G buffer");
+    static_assert(!CF::HERM || KR * LDP <= CF::KR * CF::LDP, "reduced P does not fit the P buffer");
+    static_assert(!CF::HERM || M * N + N <= M * CF::N, "reduced dv does not fit behind T21");
 };
 // Basis descriptors (ints, built once per launch from sigma, m4q_kernels.cu build_tables):
 //   coordinate a < N:  HB_J1 / HB_J2 [a]: the two realified indices it averages (equal for a fixed point; -1: padding);
@@ -127,8 +128,12 @@ template <class CF> struct Rec {
     static_assert(B % 2 == 0 && SMALL % 2 == 0 && SIZE % 2 == 0, "records are moved in 16-byte chunks");
     // offset of K[a][k] / B[k][i] (k = realified state index) inside their pair blocks
     __host__ __device__ static constexpr int pair(int ctl, int k) { return (ctl * CF::C + (k % CF::C)) * 2 + (k >= CF::C); }
-    // during the vector sweeps whole records are staged in the [P | G] buffers (only live inside the factor)
-    static_assert(SLOT + SIZE <= CF::KR * (CF::LDP + CF::LDG), "record ring does not fit the factor scratch");
+    // during the vector sweeps whole records are staged in the [P | G] buffers (only live inside the factor).  With
+    // C = 4 and three or more controls two records are longer than [P | G] (242 / 280 doubles against 224): the ring
+    // then gets a slab region of its own (Slab::layout), at least as long as [P | G] so that the exact-stage scratch,
+    // which also lives at the ring, fits either way.
+    static constexpr bool ALIAS = SLOT + SIZE <= CF::KR * (CF::LDP + CF::LDG);
+    static constexpr int OWN = cmax(SLOT + SIZE, CF::KR * (CF::LDP + CF::LDG));   // length of the ring's own region
 };
 template <class CF> __host__ __device__ constexpr int ws_doubles(int H) {
     return H * Rec<CF>::SIZE + 2 * (H + 1) * CF::N;
@@ -136,7 +141,7 @@ template <class CF> __host__ __device__ constexpr int ws_doubles(int H) {
 
 template <class CF> struct Slab {
     double *P, *AB, *W, *T21, *S, *ring, *kk, *hl, *Ug, *Uo, *z, *y, *x0, *va, *vb, *xT, *lo0, *hi0, *xcur, *xmeas, *scr;
-    double *recring;   // 2-slot ring of whole stage records for the vector sweeps (aliases the factor scratch)
+    double *recring;   // 2-slot ring of whole stage records for the vector sweeps (aliases the factor scratch if it fits)
     double *xd;        // 2 N doubles of scratch for the general-cost adjoint sweep
     int *mask;
     int *flips;        // how often a control has been released from the working set during the current QP solve
@@ -165,7 +170,7 @@ template <class CF> struct Slab {
         take(&q->AB, CF::KR * CF::LDG);      // G = [A_t | B~_t | D~_t], zero padded, [KR][LDG]
         take(&q->W, M * N);                  // K_t for the update of P (W = P G itself never leaves the registers)
         q->scr = q->AB;
-        q->recring = q->P;
+        if (Rec<CF>::ALIAS) q->recring = q->P;
         take(&q->xd, 2 * N);
         take(&q->T21, M * N);
         take(&q->S, M * M);
@@ -189,6 +194,7 @@ template <class CF> struct Slab {
         if (s) s->mask = reinterpret_cast<int *>(mk);
         take(&mk, cdiv(H * M, 2));
         if (s) s->flips = reinterpret_cast<int *>(mk);
+        if (!Rec<CF>::ALIAS) take(&q->recring, Rec<CF>::OWN, 16);
         return o;
     }
     // the part that must survive between launches in host-stepped mode: Xg | Ug | z | y | xcur | xmeas

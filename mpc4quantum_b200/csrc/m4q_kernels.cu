@@ -1955,21 +1955,25 @@ static int launch_mpc(const m4q_mpc_problem *p, long long n, const MpcArgs &base
     return 0;
 }
 
+// The compiled (c, m) instantiations: c in {4, 8, 9, 16} (qubit, stacked two-qubit, qutrit and two-qubit or process
+// vectors), one to four controls.  X(c, m, args...) is applied to each; the dispatch, m4q_supported and the workspace
+// sizes are generated from this one list.
+#define M4Q_SHAPES(X, ...)                                                                                             \
+    X(4, 1, __VA_ARGS__) X(4, 2, __VA_ARGS__) X(4, 3, __VA_ARGS__) X(4, 4, __VA_ARGS__)                                \
+    X(8, 1, __VA_ARGS__) X(8, 2, __VA_ARGS__) X(8, 3, __VA_ARGS__) X(8, 4, __VA_ARGS__)                                \
+    X(9, 1, __VA_ARGS__) X(9, 2, __VA_ARGS__) X(9, 3, __VA_ARGS__) X(9, 4, __VA_ARGS__)                                \
+    X(16, 1, __VA_ARGS__) X(16, 2, __VA_ARGS__) X(16, 3, __VA_ARGS__) X(16, 4, __VA_ARGS__)
+
+// runs the statements with CF = Cfg<c, m>, or returns the error of an unsupported pair
+#define M4Q_DISPATCH_CASE(C_, M_, c, m, ...) if ((c) == C_ && (m) == M_) { using CF = Cfg<C_, M_>; __VA_ARGS__; } else
 #define M4Q_DISPATCH(c, m, ...)                                                       \
     do {                                                                              \
-        if ((c) == 4 && (m) == 1) { using CF = Cfg<4, 1>; __VA_ARGS__; }              \
-        else if ((c) == 4 && (m) == 2) { using CF = Cfg<4, 2>; __VA_ARGS__; }         \
-        else if ((c) == 9 && (m) == 2) { using CF = Cfg<9, 2>; __VA_ARGS__; }         \
-        else if ((c) == 8 && (m) == 2) { using CF = Cfg<8, 2>; __VA_ARGS__; }         \
-        else if ((c) == 16 && (m) == 3) { using CF = Cfg<16, 3>; __VA_ARGS__; }       \
-        else if ((c) == 16 && (m) == 1) { using CF = Cfg<16, 1>; __VA_ARGS__; }       \
-        else return fail("unsupported (c, m): no compiled instantiation");            \
+        M4Q_SHAPES(M4Q_DISPATCH_CASE, c, m, __VA_ARGS__)                              \
+        return fail("unsupported (c, m): no compiled instantiation");                 \
     } while (0)
 
-static bool supported(int c, int m) {
-    return (c == 4 && m == 1) || (c == 4 && m == 2) || (c == 9 && m == 2) || (c == 8 && m == 2) || (c == 16 && m == 3) ||
-           (c == 16 && m == 1);
-}
+#define M4Q_SUPPORTED_CASE(C_, M_, c, m) || ((c) == C_ && (m) == M_)
+static bool supported(int c, int m) { return false M4Q_SHAPES(M4Q_SUPPORTED_CASE, c, m); }
 
 static int check_problem(const m4q_mpc_problem *p) {
     if (!p) return fail("null problem");
@@ -2123,18 +2127,7 @@ int m4q_exact_linearize_batched(int64_t N, int32_t c, int32_t m, int32_t H, doub
 }
 
 int64_t m4q_qp_workspace_bytes(int64_t N, int32_t c, int32_t m, int32_t H) {
-    int64_t per = -1;
-    if (c == 4 && m == 1) per = qp_ws_doubles<Cfg<4, 1>>(H);
-    else if (c == 4 && m == 2) per = qp_ws_doubles<Cfg<4, 2>>(H);
-    else if (c == 9 && m == 2) per = qp_ws_doubles<Cfg<9, 2>>(H);
-    else if (c == 8 && m == 2) per = qp_ws_doubles<Cfg<8, 2>>(H);
-    else if (c == 16 && m == 3) per = qp_ws_doubles<Cfg<16, 3>>(H);
-    else if (c == 16 && m == 1) per = qp_ws_doubles<Cfg<16, 1>>(H);
-    if (per < 0) {
-        fail("unsupported (c, m): no compiled instantiation");
-        return -1;
-    }
-    return (int64_t)sizeof(double) * N * per;
+    M4Q_DISPATCH(c, m, return (int64_t)sizeof(double) * N * qp_ws_doubles<CF>(H));
 }
 
 // with room for the pivoted-KKT workspaces of the resident warps (settings.kkt_fallback != 0)

@@ -112,8 +112,7 @@ class WrapModel:
         """Batched front end: xs [B, c, H+1] complex, us [B, m, H] -> A [B,H,c,c], B [B,H,c,m], D [B,H,c]."""
         lib = _lib.lib()
         c, m, p = self.dim_x, self.dim_u, self.polyu_dim
-        if not lib.m4q_supported(c, m):
-            raise NotImplementedError('no compiled kernel for (dim_x, dim_u) = (%d, %d)' % (c, m))
+        _lib.require_shape(c, m)
         Xg = _lib.dev(xs, np.complex128)
         Ug = _lib.dev(np.real(us), np.float64)
         nb = Xg.shape[0]

@@ -222,8 +222,7 @@ class ExactModel:
         from . import _lib
         lib = _lib.lib()
         c, m = self.dim_x, self.dim_u
-        if not lib.m4q_supported(c, m):
-            raise NotImplementedError('no compiled kernel for (dim_x, dim_u) = (%d, %d)' % (c, m))
+        _lib.require_shape(c, m)
         Xg = _lib.dev(xs, np.complex128)
         Ug = _lib.dev(np.real(us), np.float64)
         nb = Xg.shape[0]

@@ -167,8 +167,7 @@ class ClosedLoopPlan:
             wrapped = WrapModel(A_x, A_u, dim_u, order)       # validates the library size (linearize.py:23-24)
             self.c, self.m, self.p = wrapped.dim_x, dim_u, wrapped.polyu_dim
             powers = wrapped.powers
-        if not lib.m4q_supported(self.c, self.m):
-            raise NotImplementedError('no compiled kernel for (dim_x, dim_u) = (%d, %d)' % (self.c, self.m))
+        _lib.require_shape(self.c, self.m)
         self.d = int(d)
         self.H, self.S = int(clock.horizon), int(clock.n_steps)
         self.external = bool(external_plant)

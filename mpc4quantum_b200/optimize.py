@@ -37,8 +37,7 @@ def quad_program_batched(x_init, X_bm, U_bm, Q_ls, R_ls, A_ls, B_ls, Delta_ls, u
     H = H1 - 1
     Ub = _lib.dev(np.real(U_bm) if not hasattr(U_bm, 'device') else U_bm, np.float64)
     m = Ub.shape[1]
-    if not lib.m4q_supported(c, m):
-        raise NotImplementedError('no compiled kernel for (dim_x, dim_u) = (%d, %d)' % (c, m))
+    _lib.require_shape(c, m)
     xi = _lib.dev(x_init, np.complex128)
     Q = _lib.dev(Q_ls, np.complex128)
     R = _lib.dev(np.real(R_ls) if not hasattr(R_ls, 'device') else R_ls, np.float64)

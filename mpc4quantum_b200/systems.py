@@ -287,6 +287,139 @@ def config_not_gate(order=1, n_steps=50, discretize=None):
                  nominal=qubit, u0=U0.flatten())
 
 
+def _ket_op(d, i, j):
+    """|i><j| + |j><i| (symmetric part of one transition) on a d-level system."""
+    out = np.zeros((d, d), dtype=complex)
+    out[i, j] = out[j, i] = 1
+    return out
+
+
+def _y_op(d, i, j):
+    """-i |i><j| + i |j><i| (the quadrature of _ket_op)."""
+    out = np.zeros((d, d), dtype=complex)
+    out[i, j], out[j, i] = -1j, 1j
+    return out
+
+
+# (dim_x, dim_u) pairs that have a configuration in config_shape (every compiled pair the BASELINE configs leave out)
+NEW_SHAPES = ((4, 3), (4, 4), (8, 1), (8, 3), (8, 4), (9, 1), (9, 3), (9, 4), (16, 2), (16, 4))
+
+
+def config_shape(c, m, order=1, n_steps=None, discretize=None):
+    """A configuration for each pair of NEW_SHAPES, with the clock and cost conventions of the BASELINE config of the
+    same state dimension.  ``cfg['detuning']`` is the plant operator ``ensemble_shape`` perturbs with.
+
+      (4, 3)   qubit with sx/2, sy/2, sz/2 controls (config_qubit's clock, costs and 1 % detuned plant)
+      (4, 4)   transmon with X01/2, Y01/2, a^+a and X12/2 drives, observed in its qubit block (QExperiment32); the model
+               is the qubit block, where X12 does not act (config_transmon_reduced)
+      (8, 1)   two qubits under ZZ crosstalk with one global X drive, both driven to |1> (config_crosstalk)
+      (8, 3)   the same with X_A, Y_A, X_B;  (8, 4): X and Y on each qubit; qubit A to |1>, B stays in |0>
+      (9, 1)   transmon driven on the X quadrature only (config_transmon)
+      (9, 3)   transmon with X, Y and a detuning (a^+a) control;  (9, 4): qutrit with X01, Y01, X12, Y12 drives
+      (16, 2)  NOT-gate synthesis with both quadratures (config_not_gate, run for n_steps without the exit test)
+      (16, 4)  two-qubit density matrix with X and Y on each qubit under ZZ, ramped target (config_cnot)
+    """
+    if (c, m) not in NEW_SHAPES:
+        raise ValueError('no configuration for (dim_x, dim_u) = (%d, %d)' % (c, m))
+    disc = discretize or discretize_homogeneous
+    name = 'shape_%d_%d' % (c, m)
+    if c == 4 and m == 3:
+        cfg = config_qubit(order, discretize=disc)
+        wq = cfg['wq']
+        H_model = [0 * SZ, 0.5 * SX, 0.5 * SY, 0.5 * SZ]
+        cfg['model'] = _dmdc(disc([liouvillian(h) for h in H_model], cfg['clock'].dt, order), 4)
+        cfg['experiment'] = QExperiment(-0.005 * wq * SZ, H_model[1:])
+        cfg['R'] = cfg['R'][0, 0] * np.eye(3)
+        det = 0.5 * SZ
+    elif c == 4:
+        cfg = config_transmon_reduced(discretize=disc)
+        alpha = cfg['nominal']._delta
+        num = destroy(3).conj().T @ destroy(3)
+        cfg['experiment'] = QExperiment32(alpha * proj(3, 2), [0.5 * _ket_op(3, 0, 1), 0.5 * _y_op(3, 0, 1), num,
+                                                                0.5 * _ket_op(3, 1, 2)])
+        H_model = [0 * I2, 0.5 * SX, 0.5 * SY, proj(2, 1), 0 * I2]
+        cfg['model'] = _dmdc(disc([liouvillian(h) for h in H_model], cfg['clock'].dt, order), 4)
+        cfg['R'] = cfg['R'][0, 0] * np.eye(4)
+        cfg['target'] = proj(3, 1).reshape(-1)      # fidelity of the plant state, which is a qutrit
+        det = num
+    elif c == 8:
+        cfg = config_crosstalk(0.05, discretize=disc)
+        Z4 = np.zeros((4, 4), dtype=complex)
+
+        def blk(a, b):
+            return np.block([[a, Z4], [Z4, b]])
+        LX, LY = liouvillian(0.5 * SX), liouvillian(0.5 * SY)
+        XA, YA, XB, YB = (0.5 * np.kron(SX, I2), 0.5 * np.kron(SY, I2), 0.5 * np.kron(I2, SX), 0.5 * np.kron(I2, SY))
+        drives = {1: ([blk(LX, LX)], [XA + XB]), 3: ([blk(LX, Z4), blk(LY, Z4), blk(Z4, LX)], [XA, YA, XB]),
+                  4: ([blk(LX, Z4), blk(LY, Z4), blk(Z4, LX), blk(Z4, LY)], [XA, YA, XB, YB])}[m]
+        cfg['model'] = _dmdc(disc([blk(Z4, Z4)] + drives[0], cfg['clock'].dt, order), 8)
+        cfg['experiment'] = QCoupledExperiment(cfg['experiment'].H0, drives[1])
+        cfg['R'] = 1e-3 * np.eye(m)
+        if m == 1:      # one global drive flips both qubits
+            S, H = cfg['clock'].n_steps, cfg['clock'].horizon
+            target_model = np.concatenate([proj(2, 1).reshape(-1)] * 2)
+            cfg['X_targ'] = np.tile(target_model[:, None], (1, S + H + 1))
+            cfg['target'] = np.kron(proj(2, 1), proj(2, 1)).reshape(-1)
+            # both qubits start tilted the same way: with config_crosstalk's opposite tilts the first-order effects of
+            # the one drive on the two populations cancel, the first QP sits on a saddle at u = 0 and a relative
+            # perturbation of 1e-15 in the model moves the closed loop's controls by 0.25
+            r = rx(-1e-3)
+            rho = r @ proj(2, 0) @ r.conj().T
+            cfg['x0'] = np.kron(rho, rho).reshape(-1)
+        det = 0.5 * (np.kron(SZ, I2) + np.kron(I2, SZ))
+    elif c == 9:
+        cfg = config_transmon(order, discretize=disc)
+        H0 = cfg['nominal'].H_list[0]
+        HX, HY = cfg['nominal'].H_list[1:]
+        num = destroy(3).conj().T @ destroy(3)
+        H1 = {1: [HX], 3: [HX, HY, num],
+              4: [0.5 * _ket_op(3, 0, 1), 0.5 * _y_op(3, 0, 1), 0.5 * _ket_op(3, 1, 2), 0.5 * _y_op(3, 1, 2)]}[m]
+        cfg['model'] = _dmdc(disc([liouvillian(h) for h in [H0] + H1], cfg['clock'].dt, order), 9)
+        cfg['experiment'] = QExperiment(H0, H1)
+        cfg['R'] = cfg['R'][0, 0] * np.eye(m)
+        det = num
+    elif m == 2:
+        from .experiment import QProcess
+        cfg = config_not_gate(order, discretize=disc)
+        H_list = [0 * SZ, 0.5 * SX, 0.5 * SY]
+        eye2, eye4 = np.eye(2), np.eye(4)
+        As_cts = [-1j * np.kron(np.kron(h, eye2) - np.kron(eye2, h.conj()), eye4) for h in H_list]
+        cfg['model'] = _dmdc(disc(As_cts, cfg['clock'].dt, order), 16)
+        cfg['experiment'] = QProcess(H_list[0], H_list[1:])
+        cfg['U_targ'] = np.vstack([cfg['U_targ'], np.zeros_like(cfg['U_targ'])])
+        cfg['R'] = 1e-2 * np.eye(2)
+        for key in ('exit_condition', 'exit_infidelity'):
+            cfg.pop(key)
+        det = 0.5 * SZ
+    else:
+        cfg = config_cnot(n_steps=n_steps or 200, discretize=disc)
+        H0 = np.kron(SZ, SZ)
+        H1 = [np.kron(SX, I2), np.kron(SY, I2), np.kron(I2, SX), np.kron(I2, SY)]
+        cfg['model'] = _dmdc(disc([liouvillian(h) for h in [H0] + H1], cfg['clock'].dt, order), 16)
+        cfg['experiment'] = QExperiment(H0, H1)
+        cfg['R'] = 1e-3 * np.eye(4)
+        det = 0.5 * (np.kron(SZ, I2) + np.kron(I2, SZ))
+    if cfg['U_targ'].shape[0] != m:     # every control but the NOT gate's tracks zero
+        cfg['U_targ'] = np.zeros((m, cfg['U_targ'].shape[1]))
+    cfg.update(name=name, dim_u=m, order=order, detuning=det)
+    if n_steps is not None and n_steps != cfg['clock'].n_steps:
+        clock = cfg['clock']
+        new = StepClock(dt=clock.dt, horizon=clock.horizon, n_steps=n_steps)
+        new.measure_freq = clock.measure_freq
+        cfg['clock'] = new
+        cols = n_steps + clock.horizon + 1
+        cfg['X_targ'] = _fit_columns(cfg['X_targ'], cols)
+        cfg['U_targ'] = _fit_columns(cfg['U_targ'], cols - 1)
+    return cfg
+
+
+def _fit_columns(a, n):
+    """The first n columns of a, the last one repeated when a has fewer."""
+    if a.shape[1] >= n:
+        return a[:, :n]
+    return np.hstack([a, np.repeat(a[:, -1:], n - a.shape[1], axis=1)])
+
+
 def _dmdc(A_full, c):
     p = A_full.shape[1] // c - 1
     return DMDc(c, c, c * p, A_full)
@@ -377,6 +510,19 @@ def ensemble_not_gate(N, seed=ENSEMBLE_SEED, lo=None, hi=None):
     H0 = 0.5 * delta[:, None, None] * SZ[None]
     H1 = (0.5 * amp[:, None, None] * SX[None])[:, None]
     return EnsembleQExperiment(H0, H1, kind='process'), dict(delta=delta, amp=amp)
+
+
+def ensemble_shape(cfg, N, seed=ENSEMBLE_SEED, lo=None, hi=None):
+    """Ensemble of a ``config_shape`` plant: every drive amplitude scaled by a ~ U[0.9, 1.1] and a detuning
+    delta ~ U[-0.1, 0.1] sat added to H0 along ``cfg['detuning']``.
+    lo, hi: only members [lo, hi) of the N-member ensemble (same values as slicing the full draw)."""
+    rng = _Draws(seed, N, lo, hi)
+    a = rng.uniform(0.9, 1.1)
+    det = rng.uniform(-0.1, 0.1) * cfg['sat']
+    ex = cfg['experiment']
+    H0 = ex.H0[None] + det[:, None, None] * cfg['detuning'][None]
+    H1 = a[:, None, None, None] * np.stack(ex.H1_list)[None]
+    return EnsembleQExperiment(H0, H1, kind=cfg.get('kind', 'identity')), dict(amplitude_scale=a, detuning=det)
 
 
 def transmon_model_liouvillians(N, seed=ENSEMBLE_SEED + 1, dt=0.25, lo=None, hi=None):

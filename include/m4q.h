@@ -187,6 +187,10 @@ int m4q_qp_admm_batched(int64_t N, int32_t c, int32_t m, int32_t H,
                         const m4q_qp_settings *settings_host,
                         double *X_out, double *U_out, double *obj_out, int32_t *status_out, int32_t *iters_out,
                         void *workspace, void *stream);
+/* Launch geometry m4q_qp_admm_batched chooses for N instances (N <= 0: the widest launch, which sizes the KKT
+   workspaces of m4q_qp_workspace_bytes_kkt). */
+int m4q_qp_launch_info(int64_t N, int32_t c, int32_t m, int32_t H, int32_t *warps_per_cta, int32_t *ctas,
+                       int32_t *smem_bytes);
 
 /*
  * Line search of the iterative QP.  Replaces iqp_line_search (mpc.py:101-125), including its pairing of a

@@ -50,6 +50,8 @@ SIGNATURES = {
     'm4q_qp_workspace_bytes_kkt': (c_i64, [c_i64, c_i32, c_i32, c_i32]),
     'm4q_qp_admm_batched': (ct.c_int, [c_i64, c_i32, c_i32, c_i32] + [c_vp] * 9 + [c_f64, c_f64, c_i32,
                                        ct.POINTER(QPSettings)] + [c_vp] * 7),
+    'm4q_qp_launch_info': (ct.c_int, [c_i64, c_i32, c_i32, c_i32, ct.POINTER(c_i32), ct.POINTER(c_i32),
+                                      ct.POINTER(c_i32)]),
     'm4q_line_search_workspace_bytes': (c_i64, [c_i32, c_i32, c_i32]),
     'm4q_line_search_batched': (ct.c_int, [c_i64, c_i32, c_i32, c_i32] + [c_vp] * 12),
     'm4q_mpc_state_bytes': (c_i64, [ct.POINTER(MpcProblem), c_i64]),

@@ -1940,9 +1940,10 @@ __device__ __noinline__ void exact_stage(const double2 *gen, const double *u, co
         }
         __syncwarp();
     }
-    // ---- b_i: Taylor series of the augmented vector system on n_sub sub-steps (||G|| / n_sub <= 4)
-    int n_sub = (theta < 128.0) ? (int)ceil(theta * 0.25) : 32;    // also catches a non-finite generator
-    if (n_sub < 1) n_sub = 1;
+    // ---- b_i: Taylor series of the augmented vector system on n_sub sub-steps, ||G|| / n_sub <= 4 for every finite
+    // theta: a long dt or a large control costs sub-steps, not accuracy.  A non-finite generator takes one sub-step and
+    // its NaN propagates into b.  theta >= 2^33, whose count would not fit an int, also takes one; its terms overflow.
+    const int n_sub = (theta > 4.0 && theta < 0x1p33) ? (int)ceil(theta * 0.25) : 1;
     const double h = 1.0 / (double)n_sub;
     // number of terms: (theta h)^K / K! < 1e-19 (sub-step norm <= 4: K <= 36; partial sums stay below e^4)
     int K = 0;

@@ -1800,6 +1800,9 @@ static int plan(KernelT kernel, int max_warps, int slab_doubles, int shared_doub
             if (best_w != warps) {
                 warps = best_w;
                 if (residency(warps, &per_sm) != 0) return -1;
+                // Keep one CTA per SM even if two of the narrower CTAs would fit: the per-warp workspaces are sized
+                // for SMs x (one CTA of the full width), and a second CTA per SM would run warps past them.
+                per_sm = 1;
             }
         }
     }
@@ -1842,6 +1845,9 @@ template <class CF> static int mpc_geometry(const m4q_mpc_problem *p, long long 
         return plan(mpc_kernel<CF, true>, CF::MAXW, slab, mpc_shared_doubles<CF>(p->p + 1), n, have_device, g);
     return plan(mpc_kernel<CF, false>, CF::MAXW, slab, mpc_shared_doubles<CF>(p->p + 1), n, have_device, g);
 }
+
+// shared-memory slab of one warp of the standalone QP kernel
+template <class CF> static int qp_slab_doubles(int H) { return rup(Slab<CF>::doubles(H, 1, CF::C), 2); }
 
 // The index involution sigma of the lift: the model state of a Hermitian plant state satisfies x_sigma(k) = conj(x_k).
 //   identity lift, vec(rho) of a dA x dA matrix (external plant: c must be a square): transpose
@@ -2137,14 +2143,30 @@ int64_t m4q_qp_workspace_bytes_kkt(int64_t N, int32_t c, int32_t m, int32_t H) {
     long long kkt = 0;
     M4Q_DISPATCH(c, m, {
         Geometry g;
-        const int slab = rup(Slab<CF>::doubles(H, 1, CF::C), 2);
         int count = 0;
         const bool have_device = cudaGetDeviceCount(&count) == cudaSuccess && count > 0;
         if (!have_device) cudaGetLastError();
-        if (plan(qp_kernel<CF>, CF::MAXW, slab, 0, 1LL << 40, have_device, &g) != 0) return -1;
+        if (plan(qp_kernel<CF>, CF::MAXW, qp_slab_doubles<CF>(H), 0, 1LL << 40, have_device, &g) != 0) return -1;
         kkt = (long long)g.ctas * g.warps * Kkt<CF>::doubles(H);
     });
     return base + (int64_t)sizeof(double) * kkt;
+}
+
+int m4q_qp_launch_info(int64_t N, int32_t c, int32_t m, int32_t H, int32_t *warps_per_cta, int32_t *ctas,
+                       int32_t *smem_bytes) {
+    if (H < 1) return fail("QP: horizon out of range");
+    Geometry g;
+    int count = 0;
+    const bool have_device = cudaGetDeviceCount(&count) == cudaSuccess && count > 0;
+    if (!have_device) cudaGetLastError();
+    M4Q_DISPATCH(c, m, {
+        if (plan(qp_kernel<CF>, CF::MAXW, qp_slab_doubles<CF>(H), 0, N > 0 ? (long long)N : 1LL << 40, have_device, &g) != 0)
+            return -1;
+    });
+    if (warps_per_cta) *warps_per_cta = g.warps;
+    if (ctas) *ctas = g.ctas;
+    if (smem_bytes) *smem_bytes = g.smem;
+    return 0;
 }
 
 int m4q_qp_admm_batched(int64_t N, int32_t c, int32_t m, int32_t H, const double *x_init, const double *X_bm,
@@ -2180,7 +2202,7 @@ int m4q_qp_admm_batched(int64_t N, int32_t c, int32_t m, int32_t H, const double
     a.ws = (double *)workspace;
     M4Q_DISPATCH(c, m, {
         Geometry g;
-        const int slab = rup(Slab<CF>::doubles(H, 1, CF::C), 2);
+        const int slab = qp_slab_doubles<CF>(H);
         if (plan(qp_kernel<CF>, CF::MAXW, slab, 0, N, true, &g) != 0) return -1;
         a.slab_doubles = slab;
         if (a.set.kkt_mode) a.set.kkt = a.ws + (size_t)N * qp_ws_doubles<CF>(H);   // sized by m4q_qp_workspace_bytes_kkt

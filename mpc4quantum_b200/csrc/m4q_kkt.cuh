@@ -430,6 +430,7 @@ __device__ __noinline__ int kkt_active_set(SlabRef sr, const QPData &qp_in, cons
 #pragma unroll 1
         for (int e = lane; e < HM; e += 32) {
             const int t = e / M, i = e % M;
+            if (!(box_hi(s, qp.sat, t, i) > box_lo(s, qp.sat, t, i))) continue;   // pinned: see below
             const double u = s.z[e];
             comp += (u - box_lo(s, qp.sat, t, i)) * s.y[e] + (box_hi(s, qp.sat, t, i) - u) * s.hl[e];
         }
@@ -438,10 +439,14 @@ __device__ __noinline__ int kkt_active_set(SlabRef sr, const QPData &qp_in, cons
         cnt.kkt++;
         if (!kkt_solve<CF, FUSED>(sr, qp_in, kkt, lane, SIGMA * mu, false)) return 3;
         // step lengths: primal (slacks) and dual (multipliers) stay positive
+        // A zero-width box (|u_0 - u_prev| <= 0, or u_prev = sat + du) has no interior: its control stays at the box,
+        // where the solve's barrier diagonal (1e300) pins it, and its multipliers stay 1 so that the working set below
+        // holds it on its bound.  Its zero slacks would otherwise stop the primal steps and turn mu into NaN.
         double ap = 1.0, ad = 1.0;
 #pragma unroll 1
         for (int e = lane; e < HM; e += 32) {
             const int t = e / M, i = e % M;
+            if (!(box_hi(s, qp.sat, t, i) > box_lo(s, qp.sat, t, i))) continue;
             const double u = s.z[e], du = s.Uo[e] - u;
             const double sl = u - box_lo(s, qp.sat, t, i), su = box_hi(s, qp.sat, t, i) - u;
             const double zl = s.y[e], zu = s.hl[e];
@@ -456,6 +461,7 @@ __device__ __noinline__ int kkt_active_set(SlabRef sr, const QPData &qp_in, cons
 #pragma unroll 1
         for (int e = lane; e < HM; e += 32) {
             const int t = e / M, i = e % M;
+            if (!(box_hi(s, qp.sat, t, i) > box_lo(s, qp.sat, t, i))) continue;
             const double u = s.z[e], du = s.Uo[e] - u;
             const double sl = u - box_lo(s, qp.sat, t, i), su = box_hi(s, qp.sat, t, i) - u;
             const double zl = s.y[e], zu = s.hl[e];

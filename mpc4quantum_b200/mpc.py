@@ -172,6 +172,12 @@ class ClosedLoopPlan:
         self.H, self.S = int(clock.horizon), int(clock.n_steps)
         self.external = bool(external_plant)
         self.xdim = self.c if self.external else self.d * self.d
+        if fid_target is not None and not self.external:
+            # the kernel reads one target entry per plant-state entry (per entry of the lifted process vector)
+            n_fid = self.c if lift_mode == _lib.LIFT_PROCESS else self.d * self.d
+            if np.asarray(fid_target).size != n_fid:
+                raise ValueError('fid_target has %d entries, the plant state has %d'
+                                 % (np.asarray(fid_target).size, n_fid))
         X_targ = np.atleast_2d(np.asarray(X_targ, dtype=complex))
         U_targ = np.atleast_2d(np.real(np.asarray(U_targ)))
         n_targ = self.S + self.H + 1

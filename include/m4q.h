@@ -56,7 +56,8 @@ typedef struct {
                             that works for the order-1 model at H = 100, where the cost-to-go leaves the fp64 range.
                             2: the same as soon as the Riccati path breaks down numerically (a settled working set whose
                             solve is not stationary or not finite, or a rollout that grows by more than 1e3 over the
-                            horizon), and from then on for every QP of that member.
+                            horizon), and from then on for every QP of that member, across the launches of a
+                            split run too (the switch is part of the state m4q_mpc_closed_loop carries).
                             4: every QP goes to the KKT solve (no Riccati attempt): slow; for cross-checking the two
                             solvers against each other on any problem.  Needs H (2n+m)(4n+2m+2) doubles per resident warp (n = 2c), which
                             m4q_mpc_table_bytes / m4q_qp_workspace_bytes_kkt include when this is set. */
@@ -217,7 +218,12 @@ int m4q_line_search_batched(int64_t N, int32_t c, int32_t m, int32_t H,
  *   external_plant != 0 (with prob.d = 0): the kernel does not propagate the plant; xs is [N][c][S+1] and holds
  *   LIFTED model states which the caller writes into xs[:, :, step_begin] before each single-step launch
  *   (host-stepped mode for a user-defined Experiment.simulate / exit_condition; mpc.py:247-292 stay on the host).
- *   state: m4q_mpc_state_bytes(prob, N) bytes, carries guesses and ADMM duals between launches.
+ *   state: m4q_mpc_state_bytes(prob, N) bytes, carries each member between launches: per member the guesses Xg and
+ *   Ug, the ADMM duals z and y, the measured plant state and, last, one flags word (the KKT switch of
+ *   kkt_fallback = 2), so that a run split into step ranges computes what one launch computes.  A member whose exit
+ *   code is not 0 when a launch with step_begin > 0 starts is left untouched by that launch: its exit code, steps,
+ *   counters, fidelity and state keep the values of the launch it stopped in.
+ *   noise_sigma > 0 is refused for the process lift (M4Q_LIFT_PROCESS), which measures a propagator.
  *   tables: m4q_mpc_table_bytes(prob) bytes of device memory, owned by the caller, re-usable across launches of the
  *   same problem: the member-independent tables (realified costs, targets) followed by one L2-resident workspace
  *   per resident warp (stage records [K | S^-1 | dv | B | D | A_t | x - r] and the state trajectories of the member

@@ -197,10 +197,13 @@ template <class CF> struct Slab {
         if (!Rec<CF>::ALIAS) take(&q->recring, Rec<CF>::OWN, 16);
         return o;
     }
-    // the part that must survive between launches in host-stepped mode: Xg | Ug | z | y | xcur | xmeas
+    // the part of a member that must survive between launches of a split run (host-stepped mode, step ranges):
+    // Xg | Ug | z | y | xmeas (2 dd, then 2 dd unused) | flags (one 64-bit word, padded to two doubles; bit 0: the
+    // KKT switch of kkt_mode 2, Counters::sticky).  The flags come last so that the prefix keeps its offsets.
     __host__ __device__ static int persistent_doubles(int H, int dd) {
-        return (H + 1) * CF::N + 3 * H * CF::M + 4 * dd;
+        return (H + 1) * CF::N + 3 * H * CF::M + 4 * dd + 2;
     }
+    __host__ __device__ static int persistent_flags(int H, int dd) { return persistent_doubles(H, dd) - 2; }
 };
 
 // ---------------------------------------------------------------------------------------------------------
@@ -328,6 +331,7 @@ struct Counters {
     int admm, factor, polish, solves;
     int kkt;        // pivoted KKT solves (reported with the polish rounds)
     int sticky;     // kkt_mode 2: a QP of this member broke down numerically in the Riccati path; later QPs skip it
+                    // (carried across the launches of a split run in the flags word of the persistent state)
     int fac_herm, fac_full;   // factorisations in Hermitian / realified coordinates
 };
 

@@ -562,6 +562,7 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
     const int *hb = reinterpret_cast<const int *>(a.tab + L.hb);
     const bool herm_launch = CF::HERM && !EXACT && hb[HermBasis<CF>::OK] != 0;
     const int persist = Slab<CF>::persistent_doubles(H, cmax(dd, C));
+    const int flags_at = Slab<CF>::persistent_flags(H, cmax(dd, C));
 
     for (;;) {
         long long k = 0;
@@ -620,6 +621,10 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
                 s.y[e] = 0.0;
             }
         } else {
+            // a member that stopped in an earlier launch (exit code 1, 2 or 3) keeps what that launch wrote: its exit
+            // code, steps, counters, fidelity and state are left as they are
+            exit_code = a.exit_code[k];
+            if (exit_code != 0) continue;
             const double *st = a.state + (size_t)k * persist;
             int o = 0;
 #pragma unroll 1
@@ -637,7 +642,9 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
                 xcur[lane] = xs_k[(size_t)lane * (S + 1) + a.step_begin];
                 xmeas[lane] = make_double2(st[o + 2 * lane], st[o + 2 * lane + 1]);
             }
-            exit_code = a.exit_code[k];
+            // kkt_mode 2: a member that has switched to the pivoted KKT solve stays switched
+            const unsigned long long flags = *reinterpret_cast<const unsigned long long *>(st + flags_at);
+            cnt.sticky = (int)(flags & 1ull);
         }
         __syncwarp();
 
@@ -898,6 +905,11 @@ __global__ void __launch_bounds__(CF::MAXW * 32) mpc_kernel(const MpcArgs a) {
             if (lane < xdim) {
                 st[o + 2 * lane] = xmeas[lane].x;
                 st[o + 2 * lane + 1] = xmeas[lane].y;
+            }
+            if (lane == 0) {
+                unsigned long long *flags = reinterpret_cast<unsigned long long *>(st + flags_at);
+                flags[0] = cnt.sticky ? 1ull : 0ull;
+                flags[1] = 0ull;
             }
         }
         __syncwarp();
@@ -2304,6 +2316,10 @@ int m4q_mpc_closed_loop(const m4q_mpc_problem *p, int64_t N, const double *x0, i
                         int32_t external_plant, double *xs, double *us, int32_t *exit_code, int32_t *steps_done,
                         int32_t *qp_count, int32_t *counters, double *fidelity, void *state, void *tables, void *stream) {
     if (check_problem(p) != 0) return -1;
+    // the process lift measures a propagator, and the reference defines no noise model for it (QSynthesis has no
+    // set_sigma)
+    if (!external_plant && p->noise_sigma > 0 && p->lift_mode == M4Q_LIFT_PROCESS)
+        return fail("measurement noise is not defined for process (gate-synthesis) plants");
     if (N <= 0) return 0;
     if (!x0 || !xs || !us || !exit_code || !steps_done || !qp_count || !tables) return fail("null pointer");
     if (!external_plant && (!H0 || !H1)) return fail("plant Hamiltonians are required unless external_plant is set");

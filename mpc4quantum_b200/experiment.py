@@ -330,7 +330,11 @@ class EnsembleQExperiment:
 
     def set_sigma(self, sigma, seed=None):
         """Measurement noise of every member (``QExperiment.set_sigma``); the stream of member k depends on
-        (seed, global index of k, MPC step, component) only."""
+        (seed, global index of k, MPC step, component) only.  Process ensembles (gate synthesis) refuse it: their
+        plant state is a propagator, and the reference defines no measurement noise for one (QSynthesis has no
+        set_sigma)."""
+        if self.kind == 'process' and sigma:
+            raise NotImplementedError('measurement noise is not defined for process (gate-synthesis) ensembles')
         self._sigma, self._noise_seed = float(sigma), seed
 
     def simulate(self, x0, u_seg, dt, return_propagators=False):
